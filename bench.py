@@ -4,6 +4,7 @@ through ST-DBSCAN; HBM GB/s of the spoke-to-point kernel vs peak).
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's result as DIR/*.npy
 
 A step = one pass of the whole hot path (spoke-to-point + gain concat -> land persistence filter ->
 ST-DBSCAN) over one block of synthetic frames (2048 spokes x 1024 echoes x gains 40/50/75, the
@@ -77,7 +78,11 @@ def parse_args():
                     "for `value`; 0 = the workload's default")
     ap.add_argument("--cpu-frames", type=int, default=0, help="frames per CPU worker in the reference/cpu_baseline sample; 0 = the workload's default")
     ap.add_argument("--shard-profile", action="store_true", help="N>1: print per-stage wall-clock of the sharded driver to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the result of the last timed step (what "
+                    "DetectionResult.to_host() hands a caller) as float32/float64 .npy files under DIR, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[args.workload]
     args.frames_per_step = args.frames_per_step or w["frames"]
     args.e2e_frames = args.e2e_frames or w["e2e_frames"]
@@ -114,6 +119,32 @@ def load_peaks():
         d = json.loads(p.read_text())
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(host: dict, n_clusters: int, out_dir: str, suffix: str = "", budget: int = DUMP_BYTES) -> None:
+    """Write one block's result as a caller receives it (``to_host()``: points, gains, labels, frame offsets and ids, plus
+    the cluster count) to ``out_dir/<name><suffix>.npy`` in float32 / float64, so two builds can be compared output for
+    output. Per-point arrays that would exceed ``budget`` bytes are cut to a fixed, seeded sample of points, sorted, whose
+    indices are written as ``point_index``; the per-frame arrays and the cluster count are always whole."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    n = len(host["labels"])
+    per_frame = {"frame_off": np.asarray(host["frame_off"]).astype(np.float64),
+                 "frame_ids": np.asarray(host["frame_ids"]).astype(np.float64),
+                 "n_clusters": np.array([n_clusters], dtype=np.float64)}
+    point_bytes = 3 * 4 + 4 + 8 + 8                       # points, gains, labels, point_index
+    headers = 7 * 4096                                    # room for the .npy headers
+    keep = max(0, (budget - headers - sum(a.nbytes for a in per_frame.values())) // point_bytes)
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    out = {"points": np.asarray(host["points"])[idx].astype(np.float32),
+           "gains": np.asarray(host["gains"])[idx].astype(np.float32),
+           "labels": np.asarray(host["labels"])[idx].astype(np.float64),
+           "point_index": idx.astype(np.float64), **per_frame}
+    for name, a in out.items():
+        np.save(d / f"{name}{suffix}.npy", a)
 
 
 # ------------------------------------------------------------------------------------ clocks
@@ -202,8 +233,8 @@ _REF_T4 = []
 
 
 def reference_t4():
-    """The UNMODIFIED reference script ``4_temporal_object_tracker.py`` as a module, if ``__graft_entry__.build()`` has
-    installed it under ``baseline/_ref/`` (it travels to the GPU box with the snapshot), else ``None``."""
+    """The UNMODIFIED reference script ``4_temporal_object_tracker.py`` as a module, if a copy of it has been placed
+    under ``baseline/_ref/PointCloudWork/`` (git-ignored: it is not part of this repository), else ``None``."""
     if not _REF_T4:
         import importlib.util
         path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "baseline", "_ref", "PointCloudWork", "4_temporal_object_tracker.py")
@@ -501,6 +532,8 @@ def run_ours(args):
                 ms, launches = timed(lambda: pipe.run_device(echo, d_c, d_s, d_r, frame_ids), args.steps, 0, collect=keep_last)
                 c1 = clocks.mark()
     res = results[-1]
+    if args.dump_outputs:
+        dump_outputs(res.to_host(), res.n_clusters, args.dump_outputs, f"_rank{rank}" if world > 1 else "", DUMP_BYTES // world)
     n_raw, n_pts = res.raw.n, res.points.n
     echo_bytes = B * G * args.spokes * args.bins * 4
     spoke_bytes = echo_bytes + B * G * args.spokes * 12 + 16 * n_raw          # SURVEY.md 8(d), whole stage
@@ -534,7 +567,7 @@ def run_ours(args):
     if not args.no_e2e:
         Be = max(1, min(args.e2e_frames, B))
         e_ids = frame_ids[:Be]
-        e_steps = max(4, min(args.steps, 8))
+        e_steps = args.steps
         ov2 = None
         if world == 1:
             from radar_point_cloud_tracking_b200.pipeline import OverlappedPipeline

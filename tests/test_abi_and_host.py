@@ -263,27 +263,3 @@ def test_read_back_staging_views_and_copies():
     out = dv.to_pinned_host(*ts)                                    # host tensors: plain copies
     ts[1][0] = 99
     assert out[1][0] == 0 and all(np.array_equal(o[1:] if i == 1 else o, (t.numpy()[1:] if i == 1 else t.numpy())) for i, (o, t) in enumerate(zip(out, ts)))
-
-
-def test_bench_reference_arm_uses_the_unmodified_t4_and_agrees_with_the_port(monkeypatch):
-    """bench.py's CPU legs: with the reference script installed under baseline/_ref the land filter, ST-DBSCAN and Cluster
-    records are the reference's own functions; the oracle port (the fallback when the script is absent) sees the same
-    points and the same number of clusters on the same sample."""
-    import sys
-
-    import __graft_entry__ as ge
-    import bench
-    ge.install_reference()
-    monkeypatch.setattr(sys, "argv", ["bench.py", "--spokes", "192"])
-    args = bench.parse_args()
-    w = bench.WORKLOADS[args.workload]
-    prm = tuple(sorted(bench.workload_config(args)["params"].items()))
-    job = (args.seed, 0, 14, 14, args.spokes, args.bins, 0.004, tuple(w["gains"]), 1, prm)
-    monkeypatch.setattr(bench, "_REF_T4", [])
-    if bench.reference_t4() is None:
-        pytest.skip("no reference script under baseline/_ref (and no /root/reference to install it from)")
-    ref = bench.cpu_block_sample(job)
-    monkeypatch.setattr(bench, "_REF_T4", [None])
-    port = bench.cpu_block_sample(job)
-    assert ref[5] is True and port[5] is False
-    assert ref[3] == port[3] > 0 and ref[4] == port[4] > 0

