@@ -347,6 +347,33 @@ int64_t rb_arange_edges(float lo, float hi, double step, double* out, int64_t ca
 int64_t rb_stitch_components(const int64_t* keys, int64_t n_keys, const int64_t* pair_a, const int64_t* pair_b,
                              int64_t n_pairs, int64_t* table_keys, int32_t* table_ids, int64_t cap, int64_t* n_clusters);
 
+/* ---- a7 over a whole recording: ST-DBSCAN in time windows (DESIGN.md section 3.8) ----------------------------------
+ * The labels, core flags and n_clusters of rb_stdbscan on the same points with times = the frame id of each point, for
+ * any number of points (int64; no 2^31 limit on the total) and any valid choice of windows. Points are frame-ordered:
+ * frame f holds points [frame_off_host[f], frame_off_host[f+1]) of x/y/z (component d of point i at x[i*stride] ...,
+ * z NULL = 2-D). frame_ids_host float32[F]: integers, strictly increasing, magnitude < 2^24. cuts_host[n_windows+1]:
+ * frame indices, strictly increasing from 0 to F; window k owns frames [cuts[k], cuts[k+1]) and with more than one
+ * window each is at least h = floor(eps_time) frames long. Its local problem is frames [cuts[k]-h, cuts[k+1]+h), clipped
+ * to the recording; each local problem must stay under 2^31-1 points, and the scratch follows the largest one (plus one
+ * byte per point of the recording when `core` is NULL). One window is rb_stdbscan itself; with K > 1 windows every
+ * window is planned three times (cores; components; labels) and the host stitches the components in between.
+ *   hint: host, optional: a box containing every x, y, z (its time range is ignored: each window's comes from the ids);
+ *         with it no plan syncs (a box that misses a point fails the call with RB_ERR_ARG at the end).
+ *   labels int32[N] out; core uint8[N] out (optional); n_clusters host int64 out (optional).
+ * RB_ERR_ARG before any work when the ids, offsets or cuts break the rules above. Syncs. */
+int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                         const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames,
+                         const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
+                         const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters, void* stream);
+
+/* HOST function: the pairing of two run-length encodings of the SAME boundary points (rb_shard_pack_keys' zone format:
+ * keys[j] holds from position starts[j] of the zone to the next start, -1 = not a core point; starts[0] = 0) into the
+ * distinct (key_a, key_b) pairs of the core points, sorted. Cost follows the number of runs, not of points. Writes at
+ * most cap pairs and returns their total number, or a negative RB_ERR_* when the encodings disagree on which points
+ * are core points or are malformed. */
+int64_t rb_pair_zone_runs(const int64_t* keys_a, const int64_t* starts_a, int64_t n_a, const int64_t* keys_b,
+                          const int64_t* starts_b, int64_t n_b, int64_t* pair_a, int64_t* pair_b, int64_t cap);
+
 /* ---- multi-GPU: time sharding (SURVEY section 8 e) -----------------------------------------------------------------
  * One process per GPU; rank r owns a contiguous block of frames and clusters it together with a floor(eps_time)-frame
  * halo from each neighbour (radar_point_cloud_tracking_b200/sharded.py drives the protocol, DESIGN.md section 6). The

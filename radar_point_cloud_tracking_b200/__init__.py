@@ -8,6 +8,7 @@ Drop-in for the hot functions of ``4_temporal_object_tracker.py`` / ``radar_pipe
 * :mod:`.transforms`  ``polar_to_cartesian``, ``sweep_to_point_cloud``
 * :mod:`.fusion`      concat / grid-max gain fusion
 * :mod:`.pipeline`    device-resident batch pipeline (what ``bench.py`` times)
+* :mod:`.recording`   a whole recording fed block by block: one land grid, one ST-DBSCAN labelling (windowed)
 * :mod:`.sharded`     time-sharded multi-GPU driver (one process per GPU, NCCL)
 
 All compute is hand-written CUDA behind the C ABI of ``include/radarb200.h``

@@ -98,6 +98,9 @@ SIGNATURES = {
                                    c_vp, c_vp, c_vp, C.POINTER(c_i64), C.POINTER(c_i64), c_vp]),
     "rb_arange_edges": (c_i64, [c_f32, c_f32, c_f64, c_vp, c_i64]),
     "rb_stitch_components": (c_i64, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp]),
+    "rb_stdbscan_windowed": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_f64, c_f32, c_i32,
+                                     C.POINTER(StdbscanHint), c_vp, c_vp, C.POINTER(c_i64), c_vp]),
+    "rb_pair_zone_runs": (c_i64, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64]),
     "rb_comm_unique_id": (c_i32, [c_vp]),
     "rb_comm_init": (c_i32, [c_vp, c_vp, c_i32, c_i32]),
     "rb_comm_destroy": (c_i32, [c_vp]),

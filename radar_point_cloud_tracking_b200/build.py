@@ -10,7 +10,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 INCLUDE = PKG.parent / "include"
 LIB = PKG / "libradarb200.so"
-SOURCES = ["context.cu", "spoke.cu", "land.cu", "dbscan.cu", "fuse.cu", "synth.cu", "pipeline.cu", "csv.cu", "plyfmt.cu", "clusters.cu", "comm.cu", "shard.cu"]
+SOURCES = ["context.cu", "spoke.cu", "land.cu", "dbscan.cu", "fuse.cu", "synth.cu", "pipeline.cu", "csv.cu", "plyfmt.cu", "clusters.cu", "comm.cu", "shard.cu", "recording.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -49,6 +49,12 @@ enum rb_slot {
     RB_S_SHARD_IDS, RB_S_SHARD_LOCAL, RB_S_SHARD_KEYS,   // time-sharded driver: staged frame ids, local frame list, key flags / ranks
     RB_S_GROUP_TMP,         // rb_stable_group: frame offsets of its single frame
     RB_S_LAND_ORDERED,      // land accumulate, ordered path: cell ids, grouped intensities, segment table
+    RB_S_REC_FRAMES,        // windowed ST-DBSCAN: frame offsets, frame ids, hint-violation flag
+    RB_S_REC_LOCAL,         // windowed ST-DBSCAN: times, global index, keys, labels, core flags of one window
+    RB_S_REC_KEYS,          // windowed ST-DBSCAN: every window's run-length encoded zone keys
+    RB_S_REC_KEYS_BIG,      // windowed ST-DBSCAN: encodings of the windows that outgrew the capacity guess
+    RB_S_REC_TABLE,         // windowed ST-DBSCAN: the stitched key -> cluster id table
+    RB_S_REC_CORE,          // windowed ST-DBSCAN: recording-wide core flags when the caller passes none
     RB_S_COUNT
 };
 
@@ -68,6 +74,7 @@ struct rb_ctx {
     rb_dbscan_stats last_stats;
     rb_db_plan* db_plan = nullptr;   // state shared by the rb_stdbscan_* phases (dbscan.cu)
     rb_comm* comm = nullptr;         // NCCL communicator of this context (comm.cu, rb_comm_init)
+    int64_t rec_key_cap = 0;         // windowed ST-DBSCAN: zone-encoding capacity guess (largest seen, bounded; recording.cu)
     int opt_dbscan_mode = 0;         // 0 = auto, 1 = always the general algorithm, 2 = require the tight one
     int opt_spoke_mask_variant = 0;  // 0 = auto, 1 = register-staged mask kernel, 2 = require the TMA-staged one
     int spoke_last_variant = 0;      // mask kernel the last rb_spoke_to_points launched (1 / 2)
@@ -209,6 +216,9 @@ int rb_stdbscan_enqueue(rb_ctx* ctx, const float* x, const float* y, const float
                         int64_t n, double eps_space, float eps_time, int min_samples, int32_t* labels, uint8_t* core,
                         const rb_stdbscan_hint* hint, void* stream);
 int rb_stdbscan_fetch_stats(rb_ctx* ctx, int64_t* n_clusters, void* stream);
+// phases for the windowed driver (recording.cu): set every core flag right after a plan; the plan's hint-violation word
+int rb_stdbscan_set_cores_planned(rb_ctx* ctx, const uint8_t* core_in, void* stream);
+int rb_stdbscan_hint_flag(rb_ctx* ctx, const unsigned long long** flag);
 // device flag "rb_land_accumulate saw an intensity that is not a small integer" of this context (land.cu)
 int rb_land_inexact_flag(rb_ctx* ctx, int32_t** flag, cudaStream_t stream);
 // bounds of the first *n_dev points (n_dev on the device, at most n_max): no host knowledge of n needed (land.cu)

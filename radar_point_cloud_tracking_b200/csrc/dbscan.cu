@@ -1428,6 +1428,23 @@ extern "C" int rb_stdbscan_set_cores(rb_ctx* ctx, const uint8_t* core_in, void* 
     return RB_OK;
 }
 
+// rb_stdbscan_set_cores straight after a plan, without counting neighbours first: for a caller that already holds the
+// exact core flag of every point of the plan (recording.cu). Without the count phase no point is known to have no
+// neighbour at all (core state 2, which set_cores keeps): every non-core point stays a border candidate.
+int rb_stdbscan_set_cores_planned(rb_ctx* ctx, const uint8_t* core_in, void* stream_) {
+    RB_REQUIRE(ctx && ctx->db_plan && ctx->db_plan->valid, "rb_stdbscan_set_cores_planned: no plan");
+    RB_CUDA(cudaMemsetAsync(ctx->db_plan->core, 0, (size_t)ctx->db_plan->n, (cudaStream_t)stream_));
+    ctx->db_plan->have_cores = true;
+    return rb_stdbscan_set_cores(ctx, core_in, stream_);
+}
+
+// device word the last plan raises when a point or time lies outside its hint box (valid until the next plan)
+int rb_stdbscan_hint_flag(rb_ctx* ctx, const unsigned long long** flag) {
+    RB_REQUIRE(ctx && ctx->db_plan && ctx->db_plan->valid && flag, "rb_stdbscan_hint_flag: no plan");
+    *flag = ctx->db_plan->d_ctr + 4;
+    return RB_OK;
+}
+
 extern "C" int rb_stdbscan_components(rb_ctx* ctx, const int64_t* global_index, int64_t* comp_key, void* stream_) {
     RB_REQUIRE(ctx && ctx->db_plan && ctx->db_plan->valid && ctx->db_plan->have_cores, "rb_stdbscan_components: run rb_stdbscan_cores first");
     cudaStream_t stream = (cudaStream_t)stream_;
