@@ -446,6 +446,30 @@ int rb_shard_pack_keys(rb_ctx* ctx, const int64_t* key, const int64_t* gidx, int
 int rb_csv_parse_sweep(rb_ctx* ctx, const uint8_t* text, int64_t n_bytes, int n_echo_columns, int64_t max_rows,
                        uint8_t* echo, int32_t* row_start, int32_t* prefix_end, int32_t* info, void* stream);
 
+/* Many sweep CSVs per launch, in two calls with one read-back between them. text[n_bytes] (device, n_bytes < 2^31)
+ * holds W files; file w is text[file_off[w], file_off[w] + file_len[w]), file_off[w] is a multiple of 4096 and files do
+ * not overlap: file_off[w] + file_len[w] <= file_off[w + 1] (file_off, file_len: int64 device arrays; the kernels give a
+ * chunk to the last file starting at or before it, so overlapping files would get wrong row counts). Same grammar and status bits as rb_csv_parse_sweep, decided per file: a
+ * file's status never depends on its neighbours.
+ * rb_csv_sweeps_lines: chunk_base[ceil(n_bytes / 4096) + 1] (device) receives the newline scan (chunk_base[last] = all
+ * newlines), rows[w] the data rows of file w (lines minus the header), status[w] the line-level bits (lone CR, blank
+ * line, RB_CSV_CAPACITY = more lines than rows of E + 5 fields could fill; rows[w] is then 0).
+ * rb_csv_parse_sweeps: the caller reads back rows and status, sets row_base[w] = sum of rows[v < w] over the files it
+ * wants parsed (0 rows for the others; row_base[W] = n_rows) and passes n_newlines = chunk_base[last]. For row r of
+ * file w, row R = row_base[w] + r: echo[R * E + c] = Echo_c (uint8), row_start[R] / prefix_end[R] = file-relative offsets
+ * of the row and of its fifth comma, angle[R] / scale[R] = Angle and Scale as float32; gain[w] = Gain of row 0.
+ * Leading fields: Angle and Scale of every row and Gain of row 0 must be -?D+ or -?D+.D+ (Gain: -?D+, within int32) with
+ * at most 15 digits and not a negative zero; the value is the digits as an exact double divided once by 10^(fraction
+ * digits), rounded to float32 - bit for bit what pandas' C parser gives. Anything else sets RB_CSV_LEAD_FIELDS: the
+ * echoes stay valid, the caller parses that file's leading fields itself. status[w] accumulates across both calls. */
+#define RB_CSV_LEAD_FIELDS 32  /* a leading field outside the device grammar (echoes still valid)                   */
+int rb_csv_sweeps_lines(rb_ctx* ctx, const uint8_t* text, int64_t n_bytes, const int64_t* file_off, const int64_t* file_len,
+                        int n_files, int n_echo_columns, int32_t* chunk_base, int32_t* rows, int32_t* status, void* stream);
+int rb_csv_parse_sweeps(rb_ctx* ctx, const uint8_t* text, int64_t n_bytes, const int64_t* file_off, const int64_t* file_len,
+                        int n_files, int n_echo_columns, const int32_t* chunk_base, int64_t n_newlines, const int64_t* row_base,
+                        int64_t n_rows, uint8_t* echo, int32_t* row_start, int32_t* prefix_end, float* angle, float* scale,
+                        int32_t* gain, int32_t* status, void* stream);
+
 /* ---- PLY output (SURVEY section 8 f, rank 4) ------------------------------------------------------------------------
  * HOST function: appends the vertex lines of an ASCII PLY to the file at `path` - the bytes that
  * np.savetxt(fh, data, fmt="%.4f %.4f %.4f %d %d %d") writes in write_ply_fast (5_gain_fusion_ply_builder.py:370-403;

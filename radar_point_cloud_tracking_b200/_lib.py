@@ -114,6 +114,9 @@ SIGNATURES = {
     "rb_shard_local_index": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "rb_shard_pack_keys": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp]),
     "rb_csv_parse_sweep": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "rb_csv_sweeps_lines": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "rb_csv_parse_sweeps": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i32, c_i32, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                    c_vp, c_vp, c_vp]),
     "rb_ply_append_ascii": (c_i32, [C.c_char_p, c_vp, c_vp, c_vp, c_vp, c_i64]),
     "rb_synth_echo": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_i32, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "rb_set_option": (c_i32, [c_vp, C.c_char_p, c_i64]),

@@ -622,6 +622,70 @@ def csv_parse_sweep(raw, n_echo_columns: int, device=None):
     return echo[:rows], host_offs[0], host_offs[1], 0
 
 
+CSV_CHUNK = 4096                                      # files of a batch start at multiples of this (csv.cu)
+CSV_LEAD_FIELDS = 32                                  # RB_CSV_LEAD_FIELDS: leading fields outside the device grammar
+
+
+@dataclass
+class CsvBatch:
+    """What ``rb_csv_parse_sweeps`` made of a batch of W files. Host arrays except ``echo``: ``status[W]`` (RB_CSV_* bits),
+    ``rows[W]`` (rows parsed; 0 for a file with a line-level status), ``row_base[W+1]``, and per parsed row
+    ``angle`` / ``scale`` (float32) and file-relative ``row_start`` / ``prefix_end``; ``gain[W]`` = Gain of row 0.
+    ``echo`` = uint8 device ``[row_base[W], E]``: file w's sweep is ``echo[row_base[w]:row_base[w + 1]]``."""
+    status: np.ndarray
+    rows: np.ndarray
+    row_base: np.ndarray
+    echo: torch.Tensor
+    angle: np.ndarray
+    scale: np.ndarray
+    gain: np.ndarray
+    row_start: np.ndarray
+    prefix_end: np.ndarray
+
+
+def csv_parse_sweeps(text: torch.Tensor, file_off: np.ndarray, file_len: np.ndarray, n_echo_columns: int) -> CsvBatch:
+    """Parse the W files held by the uint8 device tensor ``text`` (file w = ``text[file_off[w]:file_off[w] + file_len[w]]``,
+    offsets ascending multiples of ``CSV_CHUNK``, total under 2^31 bytes): ``rb_csv_sweeps_lines``, one read-back of the
+    row counts, exact allocation, ``rb_csv_parse_sweeps``, one read-back of the statuses and leading fields."""
+    E = int(n_echo_columns)
+    fo = np.ascontiguousarray(file_off, dtype=np.int64)
+    fl = np.ascontiguousarray(file_len, dtype=np.int64)
+    W, n = len(fo), int(text.numel())
+    if len(fl) != W or E < 1 or n >= (1 << 31):
+        raise RadarB200Error("csv batch: one length per file, num_echo_columns >= 1 and under 2^31 bytes of text")
+    # every kernel attributes a chunk to the last file starting at or before it: files must not overlap
+    if W and (np.any(fo % CSV_CHUNK) or np.any(fl < 0) or fo[0] < 0 or np.any(fo[:-1] + fl[:-1] > fo[1:]) or int(fo[-1] + fl[-1]) > n):
+        raise RadarB200Error("csv batch: files must lie in the text at ascending, non-overlapping 4096-byte aligned offsets")
+    d = text.device
+    ctx = context(d.index)
+    text = _dev(text, torch.uint8, "text")
+    d_off = torch.from_numpy(fo).to(d)
+    d_len = torch.from_numpy(fl).to(d)
+    chunks = (n + CSV_CHUNK - 1) // CSV_CHUNK
+    chunk_base = torch.empty(chunks + 1, dtype=torch.int32, device=d)
+    rows_d = torch.empty(max(W, 1), dtype=torch.int32, device=d)
+    status_d = torch.empty(max(W, 1), dtype=torch.int32, device=d)
+    check(ctx.lib.rb_csv_sweeps_lines(ctx.handle, ptr(text), n, ptr(d_off), ptr(d_len), W, E, ptr(chunk_base), ptr(rows_d), ptr(status_d),
+                                      stream_ptr()), "rb_csv_sweeps_lines")
+    rows, status, n_nl = to_pinned_host(rows_d[:W], status_d[:W], chunk_base[chunks:])
+    rows = np.where(status == 0, rows, 0).astype(np.int64)        # a file with a line-level status is not parsed
+    row_base = np.concatenate([[0], np.cumsum(rows)]).astype(np.int64)
+    R = int(row_base[-1])
+    echo = torch.empty((max(R, 1), E), dtype=torch.uint8, device=d)
+    offs = torch.empty((2, max(R, 1)), dtype=torch.int32, device=d)
+    lead = torch.empty((2, max(R, 1)), dtype=torch.float32, device=d)
+    gain = torch.zeros(max(W, 1), dtype=torch.int32, device=d)
+    if R:
+        d_base = torch.from_numpy(row_base).to(d)
+        check(ctx.lib.rb_csv_parse_sweeps(ctx.handle, ptr(text), n, ptr(d_off), ptr(d_len), W, E, ptr(chunk_base), int(n_nl[0]), ptr(d_base), R,
+                                          ptr(echo), ptr(offs[0]), ptr(offs[1]), ptr(lead[0]), ptr(lead[1]), ptr(gain), ptr(status_d),
+                                          stream_ptr()), "rb_csv_parse_sweeps")
+        status, gain_h, offs_h, lead_h = to_pinned_host(status_d[:W], gain[:W], offs[:, :R], lead[:, :R])
+    else:
+        gain_h, offs_h, lead_h = np.zeros(W, np.int32), np.zeros((2, 0), np.int32), np.zeros((2, 0), np.float32)
+    return CsvBatch(status, rows, row_base, echo[:R], lead_h[0], lead_h[1], gain_h, offs_h[0], offs_h[1])
+
+
 # --------------------------------------------------------------------------------------- synthetic input
 def synth_echo(spec, first_frame: int = 0, n_frames: Optional[int] = None, device=None,
                out: Optional[torch.Tensor] = None) -> torch.Tensor:

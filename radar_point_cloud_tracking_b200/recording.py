@@ -5,6 +5,7 @@ land filtering only when more than ``land_min_frames`` frames were built, and on
 ranks over the whole recording. :class:`RecordingDetection` computes exactly that for a recording fed block by block:
 
     add_block(echo block) ...  ->  spoke-to-point per block into one device point store (echo blocks are not kept)
+    add_csv_frames(files) ...  ->  the same from sweep CSV files, parsed in batches on the device (csvbatch)
     finish()                   ->  land grid from the recording's bounds, land filter, rb_stdbscan_windowed
 
 Frame for frame and bit for bit the result equals :meth:`pipeline.DetectionPipeline.run_device` on the concatenation
@@ -15,9 +16,11 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import os
 import time
 from dataclasses import dataclass, field
-from typing import Dict, Optional, Sequence
+from pathlib import Path
+from typing import Dict, Mapping, Optional, Sequence
 
 import numpy as np
 import torch
@@ -125,6 +128,8 @@ class RecordingResult(DetectionResult):
     frames_built: int = 0
     land_ordered: bool = False                          # non-integer intensities: the ordered accumulation ran
     timings: Dict[str, float] = field(default_factory=dict)
+    frame_times: Optional[list] = None                  # per frame (timestamp, timestamp_ms) when CSV frames were added
+                                                        # (build_frame's, T4:319-323); (None, None) for block frames
 
 
 class RecordingDetection:
@@ -145,6 +150,12 @@ class RecordingDetection:
         self._b4 = None
         self._gain_cache = None
         self._finished = False
+        self._times = []                                # per frame: (timestamp, timestamp_ms)
+        self._csv_frames = False
+        self._reader = None                             # csvbatch.SweepReader: pinned slots, allocated on first use
+        #: CSV files parsed in a batch by rb_csv_parse_sweeps / read by the drop-in's per-file reader (unreadable, or
+        #: larger than batch_bytes)
+        self.csv_files: Dict[str, int] = {"batched": 0, "per_file": 0}
         self.timings: Dict[str, float] = {"spoke": 0.0}
 
     # ---- blocks -------------------------------------------------------------------------------------------------------
@@ -185,18 +196,28 @@ class RecordingDetection:
         W = F * G
         if self._gain_cache is None or self._gain_cache.numel() < W:
             self._gain_cache = torch.tensor(list(cfg.gains) * F, dtype=torch.int32, device=d)
+        base = self._n
+        off = self._spoke_append(echo.reshape(W, S, E), cos_tab, sin_tab, range_res, self._gain_cache[:W],
+                                 lambda sweep_base: dev.frame_offsets(sweep_base, F, G))
+        self._add_frames(base, off, ids, [(None, None)] * F)
+        self.timings["spoke"] += time.perf_counter() - t0
+
+    def _spoke_append(self, echo3: torch.Tensor, cos_tab, sin_tab, range_res, sweep_gain: torch.Tensor, offsets_of) -> np.ndarray:
+        """One spoke launch over ``echo3[W,S,E]`` writing straight behind the store's points, with the capacity negotiation
+        of ``run_device_staged``; folds the bounds and advances the store. Returns the host copy of
+        ``offsets_of(sweep_base)`` (point offsets from the launch's first point; its last entry = the points written)."""
+        W, S, E = echo3.shape
+        cfg = self.cfg
         cap = self.pipe._cap_hint or dev.default_capacity(W, S, E, cfg.point_stride)
         while True:
-            # the spoke stage writes straight behind the points already in the store
             self._grow(self._n + cap)
-            out = (*(t[self._n:] for t in self._store), torch.empty(W + 1, dtype=torch.int64, device=d))
-            x, y, inten, gain, sweep_base = dev.spoke_to_points_raw(echo.reshape(W, S, E), cos_tab, sin_tab, range_res,
-                                                                    self._gain_cache[:W], cfg.intensity_threshold,
-                                                                    cfg.point_stride, cap, out=out)
+            out = (*(t[self._n:] for t in self._store), torch.empty(W + 1, dtype=torch.int64, device=echo3.device))
+            x, y, inten, gain, sweep_base = dev.spoke_to_points_raw(echo3, cos_tab, sin_tab, range_res, sweep_gain,
+                                                                    cfg.intensity_threshold, cfg.point_stride, cap, out=out)
             cap = out[0].numel()
-            off_d = dev.frame_offsets(sweep_base, F, G)
+            off_d = offsets_of(sweep_base)
             b4_d = dev.bounds_counted(x, y, sweep_base[W:])
-            off, b4 = dev.to_pinned_host(off_d, b4_d)    # the block's one read-back
+            off, b4 = dev.to_pinned_host(off_d, b4_d)    # the launch's one read-back
             n = int(off[-1])
             if n <= cap:
                 break
@@ -205,11 +226,15 @@ class RecordingDetection:
         if n:
             self._b4 = b4.copy() if self._b4 is None else np.array(
                 [min(self._b4[0], b4[0]), max(self._b4[1], b4[1]), min(self._b4[2], b4[2]), max(self._b4[3], b4[3])], np.float32)
-        self._bases.append(self._n)
-        self._offs.append(off.astype(np.int64))
-        self._ids.append(ids)
         self._n += n
-        self.timings["spoke"] += time.perf_counter() - t0
+        return off
+
+    def _add_frames(self, base: int, off: np.ndarray, ids: np.ndarray, times: list) -> None:
+        """Book frames whose points start at store index ``base`` (``off`` = their offsets from there)."""
+        self._bases.append(base)
+        self._offs.append(np.asarray(off, dtype=np.int64))
+        self._ids.append(ids)
+        self._times.extend(times)
 
     def add_host_block(self, echo, angle_units, scale, frame_ids: Sequence[int]) -> None:
         """Host echoes (numpy, or a pinned torch tensor) ``[F,G,S,E]``: spoke tables from ``angle_units`` / ``scale`` as
@@ -221,6 +246,100 @@ class RecordingDetection:
         d = self.device
         self.add_block(t.to(d, non_blocking=True), torch.from_numpy(c).to(d), torch.from_numpy(s).to(d),
                        torch.from_numpy(r).to(d), frame_ids)
+
+    def add_csv_frames(self, frame_files: Sequence[Mapping[int, "os.PathLike"]], frame_ids: Optional[Sequence[int]] = None,
+                       num_echo_columns: int = 1024, batch_bytes: int = 64 << 20, readers: Optional[int] = None) -> None:
+        """Frames from sweep CSV files, with ``build_frame``'s semantics (T4:312-352) for every frame: ``frame_files[f]``
+        maps a gain to its file; sweeps are taken in ascending gain order and their points are labelled with that key (not
+        the file's Gain column); unreadable files print the reference's message and are skipped, as are empty and
+        header-only ones; a frame left without points keeps its id with zero points. ``frame_ids`` default to the index,
+        continuing the recording's ids (from 0). ``config.gains`` is not used: frames may carry any set of gains.
+
+        Files are read by ``readers`` threads into two pinned slots kept by the recording and parsed by
+        ``rb_csv_parse_sweeps`` a batch of whole frames (at most ``batch_bytes``) at a time. The slots are allocated when a
+        call first needs them and grow, never shrink, when a later call's files need more, up to that call's
+        ``batch_bytes``: only a file larger than ``batch_bytes``, or one that cannot be read, takes the drop-in's per-file
+        reader (``csv_files`` counts both kinds). What a file outside the device grammar gets instead is decided per file
+        (``csvbatch``). Spoke-to-point runs over runs of consecutive sweeps of the same spoke count and echo type,
+        appended behind the store in sweep order."""
+        from . import csvbatch
+        from .tracker import parse_timestamp
+
+        if self._finished:
+            raise RadarB200Error("add_csv_frames after finish(): start a new RecordingDetection")
+        E = int(num_echo_columns)
+        if E < 1:
+            raise RadarB200Error("num_echo_columns must be >= 1")
+        if not (csvbatch.CSV_CHUNK <= int(batch_bytes) <= csvbatch.MAX_BATCH_BYTES):
+            raise RadarB200Error(f"batch_bytes must be in [{csvbatch.CSV_CHUNK}, {csvbatch.MAX_BATCH_BYTES}]")
+        frames = [sorted((g, Path(p)) for g, p in ff.items()) for ff in frame_files]
+        if not frames:
+            if frame_ids is not None and len(frame_ids):
+                raise RadarB200Error(f"{len(frame_ids)} frame ids for 0 frames")
+            return
+        after = self._ids[-1][-1] if self._ids else None
+        if frame_ids is None:
+            frame_ids = np.arange(len(frames)) + (0 if after is None else after + 1)
+        ids = check_frame_ids(frame_ids, after)
+        if len(ids) != len(frames):
+            raise RadarB200Error(f"{len(ids)} frame ids for {len(frames)} frames")
+        times = [parse_timestamp(fr[0][1].name) if fr else (None, None) for fr in frames]        # T4:319-323
+        if self._reader is None:
+            self._reader = csvbatch.SweepReader()
+        for k in ("read", "h2d", "parse", "lead"):
+            self.timings.setdefault(k, 0.0)
+
+        def consume(fa, fb, results):
+            self._add_csv_batch(results, ids[fa:fb], times[fa:fb], E)
+
+        self._reader.run(frames, E, self.device, readers or min(8, os.cpu_count() or 1), consume, self.timings, batch_bytes)
+        self._csv_frames = True
+
+    def _add_csv_batch(self, results, ids: np.ndarray, times: list, E: int) -> None:
+        """Spoke stage of one batch of parsed frames (see :meth:`add_csv_frames`), booked as one block."""
+        from . import csvbatch
+        from .tracker import sweep_tables
+
+        t0 = time.perf_counter()
+        d, cfg = self.device, self.cfg
+        sweeps, per_frame = [], []                       # sweeps: (gain label, angle, scale, echo device tensor, batch rows)
+        for frame in results:
+            for _, r in frame:
+                self.csv_files["per_file" if r.status is None else "batched"] += 1
+            got = [(g, r.sweep, r.rows) for g, r in frame if r.sweep is not None and r.sweep[2].shape[0] > 0]
+            host = [isinstance(sw[2], np.ndarray) for _, sw, _ in got]
+            as_u8 = [sw[2].astype(np.uint8) if h else None for (_, sw, _), h in zip(got, host)]
+            exact = all(np.array_equal(u, sw[2]) for (_, sw, _), u, h in zip(got, as_u8, host) if h)
+            for (g, sw, rows), u, h in zip(got, as_u8, host):
+                if exact:                                # 0..255 integers travel as uint8 (rb_spoke_to_points_u8)
+                    echo = torch.from_numpy(u).to(d) if h else sw[2]
+                else:                                    # the frame goes through the float32 kernel
+                    echo = torch.from_numpy(np.ascontiguousarray(sw[2], np.float32)).to(d) if h else sw[2].float()
+                    rows = None
+                sweeps.append((g, sw[0], sw[1], echo, None if h else rows))
+            per_frame.append(len(got))
+        tl = time.perf_counter()
+        self.timings["lead"] += tl - t0
+        base = self._n
+        sweep_off = [np.zeros(1, np.int64)]
+        for a, b in csvbatch.sweep_runs([(sw[3].shape[0], sw[3].dtype) for sw in sweeps]):
+            run = sweeps[a:b]
+            S = run[0][3].shape[0]
+            rows = [sw[4] for sw in run]
+            if all(r is not None for r in rows) and all(rows[i][1] == rows[i + 1][0] for i in range(len(rows) - 1)):
+                # consecutive rows of the batch's echo (same storage): a view, no copy
+                echo = run[0][3].as_strided((b - a, S, E), (S * E, E, 1))
+            else:
+                echo = torch.stack([sw[3] for sw in run])
+            t1 = time.perf_counter()
+            c, s_, r = sweep_tables(np.stack([sw[1] for sw in run]), np.stack([sw[2] for sw in run]), E, cfg.angle_scale)
+            self.timings["lead"] += time.perf_counter() - t1
+            gains = torch.tensor([sw[0] for sw in run], dtype=torch.int32, device=d)
+            off = self._spoke_append(echo, *(torch.from_numpy(np.ascontiguousarray(t)).to(d) for t in (c, s_, r)), gains,
+                                     lambda sweep_base: sweep_base)
+            sweep_off.append(off[1:] + sweep_off[-1][-1])
+        self._add_frames(base, csvbatch.frame_offsets(np.concatenate(sweep_off), per_frame), ids, times)
+        self.timings["spoke"] += time.perf_counter() - tl
 
     # ---- the recording ------------------------------------------------------------------------------------------------
     def window_budget(self, n_points: int) -> int:
@@ -309,7 +428,8 @@ class RecordingDetection:
                                                          cfg.min_samples, bounds4=self._b4)
         timings["cluster"] = time.perf_counter() - t0
         return RecordingResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum, core=core, cuts=cuts,
-                               frames_built=built, land_ordered=land_ordered, timings=timings)
+                               frames_built=built, land_ordered=land_ordered, timings=timings,
+                               frame_times=list(self._times) if self._csv_frames else None)
 
     def _chunks(self, raw_off: np.ndarray):
         """Consecutive blocks grouped into frame ranges of fewer than 2^31 points (the land kernels' per-call limit)."""

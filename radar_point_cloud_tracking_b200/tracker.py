@@ -118,10 +118,6 @@ def read_sweep_csv_device(path: Path, num_echo_columns: int = NUM_ECHO_COLUMNS):
     the reference's parser, from the offsets the device returns. A file outside the device grammar (non-integer or
     > 255 echoes, ragged rows, blank lines, quotes) is handed to :func:`read_sweep_csv` whole, so it behaves exactly
     as in the reference."""
-    import io
-
-    import pandas as pd
-
     path = Path(path)
     try:
         raw = path.read_bytes()
@@ -133,17 +129,32 @@ def read_sweep_csv_device(path: Path, num_echo_columns: int = NUM_ECHO_COLUMNS):
         return read_sweep_csv(path, num_echo_columns)
     if echo.shape[0] == 0:
         return None                                               # header only / empty: df.empty (T4:197-198)
-    lead = b"\n".join(raw[a:b] for a, b in zip(row_start.tolist(), prefix_end.tolist()))
+    lead = lead_fields_pandas(raw, row_start, prefix_end, echo.shape[0])
+    if lead is None:
+        return read_sweep_csv(path, num_echo_columns)              # let the reference's parser decide (and report)
+    angle, scale, gain = lead
+    return angle, scale, echo, gain
+
+
+def lead_fields_pandas(raw, row_start: np.ndarray, prefix_end: np.ndarray, n_rows: int):
+    """The five leading fields of a file's rows, ``raw[row_start[r]:prefix_end[r]]``, through pandas (the reference's
+    parser): ``(angle f32, scale f32, gain)``, or ``None`` when pandas fails or finds another number of rows - the file
+    then goes to :func:`read_sweep_csv` whole."""
+    import io
+
+    import pandas as pd
+
+    lead = b"\n".join(bytes(raw[a:b]) for a, b in zip(row_start.tolist(), prefix_end.tolist()))
     try:
         df = pd.read_csv(io.BytesIO(lead), header=None, names=["Status", "Scale", "Range", "Gain", "Angle"], engine="c")
         gain = int(df["Gain"].iloc[0])
         angle = df["Angle"].to_numpy(np.float32)
         scale = df["Scale"].to_numpy(np.float32)
     except Exception:
-        return read_sweep_csv(path, num_echo_columns)              # let the reference's parser decide (and report)
-    if len(df) != echo.shape[0]:
-        return read_sweep_csv(path, num_echo_columns)
-    return angle, scale, echo, gain
+        return None
+    if len(df) != n_rows:
+        return None
+    return angle, scale, gain
 
 
 def sweep_tables(angle_units: np.ndarray, scale: np.ndarray, num_bins: int, angle_scale: float = ANGLE_SCALE
@@ -369,6 +380,30 @@ def st_dbscan(frames: List[RadarFrame], eps_space: float, eps_time: float, min_s
     labels, n_clusters = dev.stdbscan(batch.x, batch.y, None, times, eps_space, eps_time, min_samples, stride=1, n=batch.n)
     rec = dev.cluster_records(batch, labels, n_clusters)
     return dev.clusters_from_records(rec, [f.frame_id for f in frames], cluster_cls, frame_id_type=lambda v: v)
+
+
+# ---- whole recordings from CSV files ----------------------------------------------------------------------
+def detect_csv_frames(frame_files: Sequence[Dict[int, Path]], skip_land_filter: bool, eps_space: float, eps_time: float,
+                      min_samples: int, _cfg=None, _cluster_cls=None) -> Dict[int, List[Cluster]]:
+    """What T4:941-977 of ``run_pipeline`` computes from the grouped files - ``build_frame`` per frame (frame id = index),
+    the land filter when more than 10 frames were built, one ``st_dbscan`` - as one :class:`recording.RecordingDetection`
+    fed by :meth:`~recording.RecordingDetection.add_csv_frames`. Configuration globals as ``install`` reads them
+    (``_cfg`` = a T4 module's :func:`_module_config`). Returns ``{frame_id: [Cluster]}``."""
+    from .pipeline import DetectionConfig
+    from .recording import RecordingDetection
+
+    cfg = _cfg or _module_config()
+    if not frame_files:
+        return {}
+    dc = DetectionConfig(intensity_threshold=cfg.INTENSITY_THRESHOLD, point_stride=cfg.POINT_STRIDE, land_filter=not skip_land_filter,
+                         land_resolution=cfg.LAND_GRID_RESOLUTION, land_persistence=cfg.LAND_PERSISTENCE_THRESHOLD,
+                         land_min_intensity=cfg.LAND_MIN_INTENSITY, eps_space=eps_space, eps_time=eps_time, min_samples=min_samples)
+    rec = RecordingDetection(dc, _cuda().index)
+    rec.add_csv_frames(frame_files, num_echo_columns=cfg.NUM_ECHO_COLUMNS)
+    res = rec.finish()
+    if res.points.n == 0:
+        return {}
+    return res.clusters_by_frame(cluster_cls=_cluster_cls or Cluster)
 
 
 # ---- drop-in installation ----------------------------------------------------------------------------
