@@ -366,6 +366,21 @@ int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y, const floa
                          const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
                          const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters, void* stream);
 
+/* rb_stdbscan_windowed with the PointCloudWorkF rules: the labels, core flags and n_clusters of rb_stdbscan_wf on the
+ * same points with times = the frame id of each point, for any number of points and any valid choice of windows. Same
+ * arguments, windows, scratch and hint as rb_stdbscan_windowed, plus min_frames (>= 1). A window's components only know
+ * the part of a cluster inside its local problem, while the WF border rule compares a border point's index with the start
+ * of the WHOLE cluster (its smallest core index): between the second and third pass the host takes every cluster's start
+ * from the stitched key table and uploads it, and the third pass assigns border points with recording-wide indices and
+ * those starts (DESIGN.md section 3.8). One window is rb_stdbscan_wf itself.
+ * RB_ERR_ARG before any work when min_frames < 1, eps_time is not <= 30 (NaN included), or the ids, offsets or cuts break the rules of
+ * rb_stdbscan_windowed. Syncs. */
+int rb_stdbscan_windowed_wf(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                            const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames,
+                            const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
+                            int min_frames, const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters,
+                            void* stream);
+
 /* HOST function: the pairing of two run-length encodings of the SAME boundary points (rb_shard_pack_keys' zone format:
  * keys[j] holds from position starts[j] of the zone to the next start, -1 = not a core point; starts[0] = 0) into the
  * distinct (key_a, key_b) pairs of the core points, sorted. Cost follows the number of runs, not of points. Writes at

@@ -211,14 +211,20 @@ __device__ __forceinline__ int rb_ld_relaxed_s32(const int* p) {
 int rb_exclusive_scan_i32(rb_ctx* ctx, const int32_t* in, int32_t* out, int64_t n,
                           int32_t* total_out, cudaStream_t stream);
 
-// ST-DBSCAN without the final counter read-back (dbscan.cu); with a hint nothing in it syncs
+// ST-DBSCAN without the final counter read-back (dbscan.cu); with a hint nothing in it syncs. min_frames > 0: the
+// PointCloudWorkF variant (rb_stdbscan_wf)
 int rb_stdbscan_enqueue(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride, const float* times,
                         int64_t n, double eps_space, float eps_time, int min_samples, int32_t* labels, uint8_t* core,
-                        const rb_stdbscan_hint* hint, void* stream);
+                        const rb_stdbscan_hint* hint, void* stream, int min_frames = 0);
 int rb_stdbscan_fetch_stats(rb_ctx* ctx, int64_t* n_clusters, void* stream);
 // phases for the windowed driver (recording.cu): set every core flag right after a plan; the plan's hint-violation word
 int rb_stdbscan_set_cores_planned(rb_ctx* ctx, const uint8_t* core_in, void* stream);
 int rb_stdbscan_hint_flag(rb_ctx* ctx, const unsigned long long** flag);
+// ... and for its min_frames variant: switch the current plan to it (0 = back to the T4 rules); the WF border rule with
+// recording-wide indices gidx[plan's n] and per cluster id the smallest core index of the whole cluster, start_of
+int rb_stdbscan_set_min_frames(rb_ctx* ctx, int min_frames);
+int rb_stdbscan_assign_global(rb_ctx* ctx, const int32_t* core_label, int32_t* labels, const int64_t* gidx, const int64_t* start_of,
+                              void* stream);
 // device flag "rb_land_accumulate saw an intensity that is not a small integer" of this context (land.cu)
 int rb_land_inexact_flag(rb_ctx* ctx, int32_t** flag, cudaStream_t stream);
 // bounds of the first *n_dev points (n_dev on the device, at most n_max): no host knowledge of n needed (land.cu)

@@ -391,12 +391,16 @@ __global__ void __launch_bounds__(DB_THREADS) dbg_keyout_kernel(int n, const uin
 // WF border rule (FIFO expansion of stdbscan_denoising_pipeline.py:337-366, see oracle st_dbscan_wf_canonical): the
 // cluster of a core neighbour q may be joined only if it started before the border point was looked at (its start
 // point = smallest core index = comp_key < the border point's index) or q IS the start point.
+// gidx / start_of (WF only, both or neither): the points are a window of a longer recording (recording.cu). Indices are
+// then the recording-wide gidx[local index], and a cluster's start is start_of[its id] - the smallest core index of the
+// WHOLE cluster, which the window's own component (comp_key) need not contain.
 template <int DIM, bool WF>
 __global__ void __launch_bounds__(DB_THREADS) dbg_border_kernel(Sorted s, DbGrid g, double eps2, float eps_t,
                                                                const uint8_t* __restrict__ core, const int* __restrict__ slabel,
                                                                const int* __restrict__ sidx, const long long* __restrict__ comp_key,
                                                                const int* __restrict__ open_list, const int* __restrict__ n_open,
-                                                               int32_t* __restrict__ labels, unsigned long long* __restrict__ ctr) {
+                                                               int32_t* __restrict__ labels, unsigned long long* __restrict__ ctr,
+                                                               const long long* __restrict__ gidx, const long long* __restrict__ start_of) {
     // one thread per LISTED point (core == 0: not core, not alone); everything else got its label from the gather kernel
     const int total = *n_open;
     unsigned long long tests = 0;
@@ -410,8 +414,8 @@ __global__ void __launch_bounds__(DB_THREADS) dbg_border_kernel(Sorted s, DbGrid
                 if (lq < best) {                          // only a smaller id can change the answer
                     if (WF) {
                         const int oq = sidx[q];
-                        const long long start = comp_key[oq];
-                        if (!(start < (long long)sidx[p] || start == (long long)oq)) return true;
+                        const long long start = start_of ? start_of[lq] : comp_key[oq];
+                        if (!(start < point_key(gidx, sidx[p]) || start == point_key(gidx, oq))) return true;
                     }
                     ++tests;
                     if (is_neighbour<DIM>(a, load_pt<DIM>(s, q), eps2, eps_t)) best = lq;
@@ -944,13 +948,15 @@ __global__ void __launch_bounds__(DB_THREADS) db_gather_labels_kernel(int n, con
 // over the window's rows: no faster (0.31 ms per 1024-frame block) - 25 lanes search at once where the serial walk stops
 // at the first bucket of cluster 0, 4.9 M instead of 1.2 M tests. The dense list with the serial early-exit walk keeps
 // both: full warps and few tests.)
+// gidx / start_of: as in dbg_border_kernel (WF only; the start of a bucket's cluster is then start_of[b_label[b]]).
 template <int DIM, bool WF>
 __global__ void __launch_bounds__(DB_THREADS) dbt_border_kernel(Sorted s, DbGrid g, double eps2, const uint8_t* __restrict__ core,
                                                                const int* __restrict__ sidx, const int* __restrict__ open_list,
                                                                const int* __restrict__ n_open, const int* __restrict__ b_ncore,
                                                                const int* __restrict__ core_start, const int* __restrict__ b_label,
                                                                const int* __restrict__ b_parent, const long long* __restrict__ b_minkey,
-                                                               int32_t* __restrict__ labels, unsigned long long* __restrict__ ctr) {
+                                                               int32_t* __restrict__ labels, unsigned long long* __restrict__ ctr,
+                                                               const long long* __restrict__ gidx, const long long* __restrict__ start_of) {
     const int total = *n_open;
     const int per_t = g.n[0] * g.n[1] * g.n[2];
     unsigned long long tests = 0;
@@ -960,7 +966,8 @@ __global__ void __launch_bounds__(DB_THREADS) dbt_border_kernel(Sorted s, DbGrid
         const CellPos c = decode_cell(g, cell);
         const Window w = window_of<DIM>(g, c);
         const int sp = cell - c.tb * per_t;
-        const long long me = sidx[p];
+        const int orig = sidx[p];
+        const long long me = WF ? point_key(gidx, orig) : orig;
         int best = INT_MAX;
         for (int tt = w.t0; tt <= w.t1; ++tt) {
             const int b = tt * per_t + sp;
@@ -968,9 +975,9 @@ __global__ void __launch_bounds__(DB_THREADS) dbt_border_kernel(Sorted s, DbGrid
             if (WF) {
                 // WF border rule: the bucket's cluster must have started before this point was looked at, or its start
                 // point itself (the core whose index is the component key) must be among the neighbours
-                const long long start = b_minkey[b_parent[b]];
+                const long long start = start_of ? start_of[b_label[b]] : b_minkey[b_parent[b]];
                 bool ok = start < me;
-                for (int q = s.cell_start[b]; !ok && q < s.cell_start[b + 1]; ++q) ok = core[q] == 1 && (long long)sidx[q] == start;
+                for (int q = s.cell_start[b]; !ok && q < s.cell_start[b + 1]; ++q) ok = core[q] == 1 && point_key(gidx, sidx[q]) == start;
                 if (!ok) continue;
             }
             best = min(best, b_label[b]);
@@ -987,17 +994,17 @@ __global__ void __launch_bounds__(DB_THREADS) dbt_border_kernel(Sorted s, DbGrid
                             if (b_ncore[b] == 0 || (xx == c.cx && yy == c.cy && zz == c.cz)) continue;
                             const int lb = b_label[b];
                             if (lb >= best) continue;                 // only a smaller id can change the answer
-                            const long long start = WF ? b_minkey[b_parent[b]] : 0;
+                            const long long start = WF ? (start_of ? start_of[lb] : b_minkey[b_parent[b]]) : 0;
                             const bool any_core = !WF || start < me;   // WF: else only the start point itself counts
                             for (int q = s.cell_start[b]; q < s.cell_start[b + 1]; ++q) {
-                                if (core[q] != 1 || (!any_core && (long long)sidx[q] != start)) continue;
+                                if (core[q] != 1 || (!any_core && point_key(gidx, sidx[q]) != start)) continue;
                                 ++tests;
                                 if (near_enough<DIM>(a, load_pt<DIM>(s, q), eps2)) { best = lb; break; }
                             }
                         }
                     }
         }
-        if (best != INT_MAX) labels[me] = best;
+        if (best != INT_MAX) labels[orig] = best;
     }
     add_counter(ctr, tests);
 }
@@ -1316,8 +1323,10 @@ int phase_components(rb_ctx* ctx, rb_db_plan& P, const long long* gidx, cudaStre
     return RB_OK;
 }
 
+// gidx / start_of: see dbg_border_kernel (read only by the WF border rule)
 template <int DIM>
-int phase_assign(rb_ctx* ctx, rb_db_plan& P, const int32_t* core_label, int32_t* labels, cudaStream_t stream) {
+int phase_assign(rb_ctx* ctx, rb_db_plan& P, const int32_t* core_label, int32_t* labels, const long long* gidx, const long long* start_of,
+                 cudaStream_t stream) {
     const int n = P.n;
     const unsigned blocks = (unsigned)rb_div_up(n, DB_THREADS);
     const Sorted s = sorted_view(P);
@@ -1332,16 +1341,17 @@ int phase_assign(rb_ctx* ctx, rb_db_plan& P, const int32_t* core_label, int32_t*
     const unsigned wblocks = (unsigned)(blocks < (unsigned)ctx->sm_count * 8 ? blocks : (unsigned)ctx->sm_count * 8);
     if (P.g.tight && wf)
         RB_CUDA(rb_launch(ctx, dbt_border_kernel<DIM, true>, dim3(wblocks), dim3(DB_THREADS), 0, stream, s, P.g, P.eps2, P.core, P.sidx, open_list, n_open,
-                          P.b_ncore, P.core_start, P.b_label, P.b_parent, P.b_minkey, labels, P.d_ctr + 2));
+                          P.b_ncore, P.core_start, P.b_label, P.b_parent, P.b_minkey, labels, P.d_ctr + 2, gidx, start_of));
     else if (P.g.tight)
         RB_CUDA(rb_launch(ctx, dbt_border_kernel<DIM, false>, dim3(wblocks), dim3(DB_THREADS), 0, stream, s, P.g, P.eps2, P.core, P.sidx, open_list, n_open,
-                          P.b_ncore, P.core_start, P.b_label, P.b_parent, P.b_minkey, labels, P.d_ctr + 2));
+                          P.b_ncore, P.core_start, P.b_label, P.b_parent, P.b_minkey, labels, P.d_ctr + 2, (const long long*)nullptr,
+                          (const long long*)nullptr));
     else if (wf)
         RB_CUDA(rb_launch(ctx, dbg_border_kernel<DIM, true>, dim3(wblocks), dim3(DB_THREADS), 0, stream, s, P.g, P.eps2, P.eps_t, P.core, P.slabel, P.sidx,
-                          P.comp_key, open_list, n_open, labels, P.d_ctr + 2));
+                          P.comp_key, open_list, n_open, labels, P.d_ctr + 2, gidx, start_of));
     else
         RB_CUDA(rb_launch(ctx, dbg_border_kernel<DIM, false>, dim3(wblocks), dim3(DB_THREADS), 0, stream, s, P.g, P.eps2, P.eps_t, P.core, P.slabel, P.sidx,
-                          P.comp_key, open_list, n_open, labels, P.d_ctr + 2));
+                          P.comp_key, open_list, n_open, labels, P.d_ctr + 2, (const long long*)nullptr, (const long long*)nullptr));
     RB_LAUNCH_CHECK(ctx);
     return RB_OK;
 }
@@ -1459,7 +1469,27 @@ extern "C" int rb_stdbscan_assign(rb_ctx* ctx, const int32_t* core_label, int32_
     RB_REQUIRE(core_label && labels, "NULL argument");
     cudaStream_t stream = (cudaStream_t)stream_;
     rb_db_plan& P = *ctx->db_plan;
-    return DB_DISPATCH(P, phase_assign)(ctx, P, core_label, labels, stream);
+    return DB_DISPATCH(P, phase_assign)(ctx, P, core_label, labels, nullptr, nullptr, stream);
+}
+
+// rb_stdbscan_assign for a window of a longer recording under the WF border rule (recording.cu): gidx = recording-wide
+// index of every point of the plan, start_of = per final cluster id the smallest core index of the whole cluster
+int rb_stdbscan_assign_global(rb_ctx* ctx, const int32_t* core_label, int32_t* labels, const int64_t* gidx, const int64_t* start_of,
+                              void* stream_) {
+    RB_REQUIRE(ctx && ctx->db_plan && ctx->db_plan->valid && ctx->db_plan->have_cores, "rb_stdbscan_assign_global: no cores");
+    RB_REQUIRE(ctx->db_plan->min_frames > 0, "rb_stdbscan_assign_global: the plan does not run the min_frames variant");
+    RB_REQUIRE(core_label && labels && gidx && start_of, "NULL argument");
+    rb_db_plan& P = *ctx->db_plan;
+    return DB_DISPATCH(P, phase_assign)(ctx, P, core_label, labels, (const long long*)gidx, (const long long*)start_of,
+                                        (cudaStream_t)stream_);
+}
+
+// switches the current plan to the PointCloudWorkF variant (min_frames core test + FIFO border rule) until the next plan
+int rb_stdbscan_set_min_frames(rb_ctx* ctx, int min_frames) {
+    RB_REQUIRE(ctx && ctx->db_plan && ctx->db_plan->valid, "rb_stdbscan_set_min_frames: no plan");
+    RB_REQUIRE(min_frames >= 0, "min_frames must be >= 0");
+    ctx->db_plan->min_frames = min_frames;
+    return RB_OK;
 }
 
 extern "C" int rb_relabel(rb_ctx* ctx, const int64_t* keys, int64_t n, const int64_t* table_keys, const int32_t* table_ids,
@@ -1475,13 +1505,15 @@ extern "C" int rb_relabel(rb_ctx* ctx, const int64_t* keys, int64_t n, const int
     return RB_OK;
 }
 
-// everything of rb_stdbscan except reading the counters back: with a hint nothing here syncs
+// everything of rb_stdbscan (min_frames > 0: of rb_stdbscan_wf) except reading the counters back: with a hint nothing
+// here syncs
 int rb_stdbscan_enqueue(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride, const float* times,
                         int64_t n, double eps_space, float eps_time, int min_samples, int32_t* labels, uint8_t* core,
-                        const rb_stdbscan_hint* hint, void* stream_) {
+                        const rb_stdbscan_hint* hint, void* stream_, int min_frames) {
     cudaStream_t stream = (cudaStream_t)stream_;
     RB_TRY(rb_stdbscan_plan_hinted(ctx, x, y, z, stride, times, n, eps_space, eps_time, min_samples, hint, stream_));
     rb_db_plan& P = *ctx->db_plan;
+    if (min_frames > 0) P.min_frames = min_frames;
     RB_TRY(rb_stdbscan_cores(ctx, core, stream_));
     RB_TRY(rb_stdbscan_components(ctx, nullptr, nullptr, stream_));
     // canonical numbering: rank of every component's smallest core index
@@ -1522,20 +1554,8 @@ extern "C" int rb_stdbscan_wf(rb_ctx* ctx, const float* x, const float* y, const
     if (n_clusters) *n_clusters = 0;
     if (n == 0) return RB_OK;
     RB_REQUIRE(labels, "labels is NULL");
-    cudaStream_t stream = (cudaStream_t)stream_;
-    RB_TRY(rb_stdbscan_plan(ctx, x, y, z, stride, times, n, eps_space, eps_time, min_samples, stream_));
-    rb_db_plan& P = *ctx->db_plan;
-    P.min_frames = min_frames;                                  // switches the core test and the border rule
-    RB_TRY(rb_stdbscan_cores(ctx, core, stream_));
-    RB_TRY(rb_stdbscan_components(ctx, nullptr, nullptr, stream_));
-    const unsigned blocks = (unsigned)rb_div_up(P.n, DB_THREADS);
-    RB_CUDA(rb_launch(ctx, db_rootflag_kernel, dim3(blocks), dim3(DB_THREADS), 0, stream, P.n, P.comp_key, P.flags));
-    RB_LAUNCH_CHECK(ctx);
-    int* d_total = (int*)(P.d_ctr + 3);
-    RB_TRY(rb_exclusive_scan_i32(ctx, P.flags, P.rank, P.n, d_total, stream));
-    RB_CUDA(rb_launch(ctx, db_rank_labels_kernel, dim3(blocks), dim3(DB_THREADS), 0, stream, P.n, P.comp_key, P.rank, labels));
-    RB_LAUNCH_CHECK(ctx);
-    RB_TRY(rb_stdbscan_assign(ctx, labels, labels, stream_));
+    RB_TRY(rb_stdbscan_enqueue(ctx, x, y, z, stride, times, n, eps_space, eps_time, min_samples, labels, core, nullptr, stream_,
+                               min_frames));                    // min_frames switches the core test and the border rule
     return rb_stdbscan_fetch_stats(ctx, n_clusters, stream_);
 }
 

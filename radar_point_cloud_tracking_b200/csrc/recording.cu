@@ -9,6 +9,9 @@
 //   3. plan + set_cores + components + rb_relabel with the stitched key -> id table + assign; the owned labels are copied
 // Between passes 2 and 3 the host ties the zones of neighbouring windows together (rb_pair_zone_runs) and numbers the
 // components (rb_stitch_components). One window is rb_stdbscan itself: one plan, no stitch.
+// rb_stdbscan_windowed_wf runs the same passes with the PointCloudWorkF rules (rb_stdbscan_wf): every plan is switched to
+// the min_frames core test, and pass 3 assigns border points with recording-wide indices and each cluster's recording-wide
+// start, taken from the stitched table.
 #include <math.h>
 
 #include <algorithm>
@@ -95,12 +98,14 @@ extern "C" int64_t rb_pair_zone_runs(const int64_t* keys_a, const int64_t* start
     return m;
 }
 
-extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
-                                    const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames,
-                                    const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
-                                    const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters, void* stream_) {
+namespace {
+
+// rb_stdbscan_windowed (min_frames = 0) and rb_stdbscan_windowed_wf (min_frames >= 1, checked by the caller)
+int windowed(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride, const int64_t* frame_off_host,
+             const float* frame_ids_host, int64_t n_frames, const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time,
+             int min_samples, int min_frames, const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters,
+             void* stream_) {
     // ---- input checks first (host arrays only): nothing is enqueued for a call that fails them ---------------------
-    if (n_clusters) *n_clusters = 0;
     RB_REQUIRE(n_frames >= 1 && frame_off_host && frame_ids_host, "need at least one frame, its offsets and ids");
     RB_REQUIRE(n_windows >= 1 && cuts_host, "need at least one window");
     RB_REQUIRE(frame_off_host[0] == 0, "frame offsets must start at 0");
@@ -161,7 +166,7 @@ extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y,
         RB_TRY(rb_expand_frame_times(ctx, d_off, d_ids, n_frames, N, times, stream_));
         rb_stdbscan_hint hw;
         RB_TRY(rb_stdbscan_enqueue(ctx, x, y, z, stride, times, N, eps_space, eps_time, min_samples, labels, core, window_hint(win[0], &hw),
-                                   stream_));
+                                   stream_, min_frames));
         int64_t ncl = 0;
         RB_TRY(rb_stdbscan_fetch_stats(ctx, &ncl, stream_));         // syncs; fails if the caller's box missed a point
         if (n_clusters) *n_clusters = ncl;
@@ -197,6 +202,7 @@ extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y,
         const int64_t s = w.L * stride;
         RB_TRY(rb_stdbscan_plan_hinted(ctx, x + s, y ? y + s : nullptr, z ? z + s : nullptr, stride, t_loc, w.R - w.L, eps_space, eps_time,
                                        min_samples, window_hint(w, &hw), stream_));
+        if (min_frames > 0) RB_TRY(rb_stdbscan_set_min_frames(ctx, min_frames));
         const unsigned long long* bad;
         RB_TRY(rb_stdbscan_hint_flag(ctx, &bad));
         RB_CUDA(rb_launch(ctx, rec_flag_or_kernel, dim3(1), dim3(1), 0, stream, bad, d_bad));
@@ -327,13 +333,23 @@ extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y,
     const int64_t m = rb_stitch_components(all_keys.data(), n_keys, pa.data(), pb.data(), (int64_t)pa.size(), tkeys.data(), tids.data(),
                                            (int64_t)tkeys.size(), &ncl);
     if (m < 0) return (int)m;
+    // min_frames: the start of every cluster (its smallest core index over the whole recording) for the WF border rule.
+    // A window's component key is the smallest core index of the part of the cluster inside its local problem; the
+    // cluster's start can lie outside it. The start is a core point, so it is its own key in the window that owns it;
+    // every other key of the cluster is larger, and the table is sorted by key: the first entry of each id.
+    const int64_t n_start = min_frames > 0 ? ncl : 0;
+    std::vector<int64_t> start_of((size_t)std::max<int64_t>(n_start, 1), -1);
+    for (int64_t i = 0; i < m && n_start; ++i)
+        if (start_of[(size_t)tids[(size_t)i]] < 0) start_of[(size_t)tids[(size_t)i]] = tkeys[(size_t)i];
     int64_t* d_tkeys;
-    RB_TRY(scratch_as(ctx, RB_S_REC_TABLE, (size_t)(m + m / 2 + 1), &d_tkeys));
+    RB_TRY(scratch_as(ctx, RB_S_REC_TABLE, (size_t)(m + m / 2 + 1 + n_start), &d_tkeys));
     int32_t* d_tids = (int32_t*)(d_tkeys + m);
+    int64_t* d_start = d_tkeys + m + m / 2 + 1;
     if (m) {
         RB_CUDA(cudaMemcpyAsync(d_tkeys, tkeys.data(), sizeof(int64_t) * (size_t)m, cudaMemcpyHostToDevice, stream));
         RB_CUDA(cudaMemcpyAsync(d_tids, tids.data(), sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice, stream));
     }
+    if (n_start) RB_CUDA(cudaMemcpyAsync(d_start, start_of.data(), sizeof(int64_t) * (size_t)n_start, cudaMemcpyHostToDevice, stream));
 
     // ---- pass 3: final labels of the owned points ---------------------------------------------------------------------
     for (const Window& w : win) {
@@ -344,7 +360,8 @@ extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y,
         RB_TRY(rb_stdbscan_set_cores_planned(ctx, core_all + w.L, stream_));
         RB_TRY(rb_stdbscan_components(ctx, g_loc, k_loc, stream_));
         RB_TRY(rb_relabel(ctx, k_loc, n_loc, d_tkeys, d_tids, m, cl_loc, stream_));
-        RB_TRY(rb_stdbscan_assign(ctx, cl_loc, lab_loc, stream_));
+        if (min_frames > 0) RB_TRY(rb_stdbscan_assign_global(ctx, cl_loc, lab_loc, g_loc, d_start, stream_));
+        else RB_TRY(rb_stdbscan_assign(ctx, cl_loc, lab_loc, stream_));
         RB_CUDA(cudaMemcpyAsync(labels + w.A, lab_loc + (w.A - w.L), sizeof(int32_t) * (size_t)(w.B - w.A), cudaMemcpyDeviceToDevice, stream));
     }
     unsigned long long bad = 0;
@@ -357,4 +374,27 @@ extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y,
     if (n_clusters) *n_clusters = ncl;
     if (!ctx->retired.empty()) rb_trim(ctx);
     return RB_OK;
+}
+
+}  // namespace
+
+extern "C" int rb_stdbscan_windowed(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                                    const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames,
+                                    const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
+                                    const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters, void* stream_) {
+    if (n_clusters) *n_clusters = 0;
+    return windowed(ctx, x, y, z, stride, frame_off_host, frame_ids_host, n_frames, cuts_host, n_windows, eps_space, eps_time, min_samples,
+                    0, hint, labels, core, n_clusters, stream_);
+}
+
+extern "C" int rb_stdbscan_windowed_wf(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                                       const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames,
+                                       const int64_t* cuts_host, int64_t n_windows, double eps_space, float eps_time, int min_samples,
+                                       int min_frames, const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters,
+                                       void* stream_) {
+    if (n_clusters) *n_clusters = 0;
+    RB_REQUIRE(min_frames >= 1, "min_frames must be >= 1");
+    RB_REQUIRE(eps_time <= 30.f, "rb_stdbscan_windowed_wf needs eps_time <= 30 (the frame set of a neighbourhood is a 64-bit mask)");
+    return windowed(ctx, x, y, z, stride, frame_off_host, frame_ids_host, n_frames, cuts_host, n_windows, eps_space, eps_time, min_samples,
+                    min_frames, hint, labels, core, n_clusters, stream_);
 }

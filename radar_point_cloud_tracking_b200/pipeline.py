@@ -39,6 +39,23 @@ class DetectionConfig:
     min_samples: int = trk.MIN_SAMPLES
     angle_scale: float = trk.ANGLE_SCALE
     cluster_3d: bool = False                     # cluster on (x, y, z = intensity) like 3_stdbscan_point_clouds.py (T3:177)
+    #: None: the T4 clustering. k >= 1: the PointCloudWorkF variant (stdbscan_denoising_pipeline.py:264-369, rb_stdbscan_wf):
+    #: a core point's neighbours must also cover at least k distinct frames, and its order-dependent border rule
+    min_frames: Optional[int] = None
+
+    def __post_init__(self):
+        self.validate()
+
+    def validate(self) -> None:
+        """Raises :class:`RadarB200Error` when ``min_frames`` is set but not an int >= 1, or ``eps_time`` exceeds 30 with it
+        (the variant keeps a neighbourhood's frames in a 64-bit mask)."""
+        mf = self.min_frames
+        if mf is None:
+            return
+        if isinstance(mf, bool) or not isinstance(mf, (int, np.integer)) or mf < 1:
+            raise RadarB200Error(f"min_frames must be None or an int >= 1, not {mf!r}")
+        if not float(np.float32(self.eps_time)) <= 30.0:
+            raise RadarB200Error("min_frames needs eps_time <= 30")
 
 
 @dataclass
@@ -119,6 +136,7 @@ class DetectionPipeline:
         if not torch.cuda.is_available():
             raise RadarB200Error("no CUDA device: the radar-b200 detection path is GPU only (no CPU fallback)")
         self.cfg = config or DetectionConfig()
+        self.cfg.validate()
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else device)
         self.ctx = context(self.device.index)
         self._cap_hint = 0
@@ -147,7 +165,8 @@ class DetectionPipeline:
         """``echo[F,G,S,E]`` float32 (or uint8: the radar's native 0..255 echoes, identical results, a quarter of
         the bytes) already on the device; tables ``[F*G,S]`` on the device.
         One library call (``rb_detect_block``): every launch and the small read-backs in between happen in the
-        native driver, not in Python."""
+        native driver, not in Python. With ``config.min_frames`` set the block is detected without clustering and the
+        filtered points are then labelled by ``rb_stdbscan_wf`` (times = frame ids)."""
         from . import _lib
 
         cfg = self.cfg
@@ -163,7 +182,8 @@ class DetectionPipeline:
                                 land_filter=int(bool(cfg.land_filter)), land_min_frames=int(cfg.land_min_frames),
                                 land_resolution=float(cfg.land_resolution), land_persistence=float(cfg.land_persistence),
                                 land_min_intensity=float(cfg.land_min_intensity), eps_space=float(cfg.eps_space),
-                                eps_time=float(np.float32(cfg.eps_time)), min_samples=int(cfg.min_samples), cluster=int(bool(cluster)),
+                                eps_time=float(np.float32(cfg.eps_time)), min_samples=int(cfg.min_samples),
+                                cluster=int(bool(cluster) and cfg.min_frames is None),
                                 cluster_3d=int(bool(cfg.cluster_3d)))
         cap = self._cap_hint or dev.default_capacity(F * G, S, E, cfg.point_stride)
         echo3 = echo.view(F * G, S, E)
@@ -189,7 +209,17 @@ class DetectionPipeline:
             edges = (t["x_edges"][:res.n_x_edges].copy(), t["y_edges"][:res.n_y_edges].copy())
             count, isum, land = (t[k][:nx * ny].view(nx, ny) for k in ("count", "isum", "land"))
         labels = t["labels"][:n_pts] if (cluster and n_pts > 0) else torch.empty(0, dtype=torch.int32, device=d)
-        return DetectionResult(ids, raw, pts, labels, int(res.n_clusters), land, edges, count, isum)
+        n_clusters = int(res.n_clusters)
+        if cluster and n_pts > 0 and cfg.min_frames is not None:
+            labels, n_clusters = self._cluster_wf(pts, ids)
+        return DetectionResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum)
+
+    def _cluster_wf(self, pts: dev.PointBatch, ids: np.ndarray):
+        """``rb_stdbscan_wf`` (``config.min_frames``) on a block's filtered points, times = their frame ids."""
+        cfg = self.cfg
+        times = dev.expand_frame_times(pts.frame_off, torch.from_numpy(ids.astype(np.float32)).to(pts.x.device), pts.n)
+        return dev.stdbscan(pts.x, pts.y, pts.inten if cfg.cluster_3d else None, times, cfg.eps_space, cfg.eps_time,
+                            cfg.min_samples, stride=1, n=pts.n, min_frames=cfg.min_frames)
 
     def run_device_staged(self, echo: torch.Tensor, cos_tab: torch.Tensor, sin_tab: torch.Tensor, range_res: torch.Tensor,
                           frame_ids: Optional[Sequence[int]] = None, cluster: bool = True) -> DetectionResult:
@@ -224,7 +254,7 @@ class DetectionPipeline:
         if cluster and pts.n > 0:
             times = dev.expand_frame_times(pts.frame_off, torch.from_numpy(ids.astype(np.float32)).to(d), pts.n)
             labels, n_clusters = dev.stdbscan(pts.x, pts.y, pts.inten if cfg.cluster_3d else None, times, cfg.eps_space,
-                                              cfg.eps_time, cfg.min_samples, stride=1, n=pts.n)
+                                              cfg.eps_time, cfg.min_samples, stride=1, n=pts.n, min_frames=cfg.min_frames)
         return DetectionResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum)
 
     # ---- host entry (the call a user of the reference makes with parsed sweeps) -----------------

@@ -10,7 +10,8 @@ ranks over the whole recording. :class:`RecordingDetection` computes exactly tha
 
 Frame for frame and bit for bit the result equals :meth:`pipeline.DetectionPipeline.run_device` on the concatenation
 of all blocks as one block. Clustering runs in time windows (DESIGN.md section 3.8) when the filtered points do not fit
-one ST-DBSCAN call; ``max_window_points`` forces smaller windows.
+one ST-DBSCAN call; ``max_window_points`` forces smaller windows. With ``DetectionConfig.min_frames`` set the labelling is
+the PointCloudWorkF variant (``rb_stdbscan_windowed_wf``), equal to ``rb_stdbscan_wf`` on the filtered points.
 """
 from __future__ import annotations
 
@@ -90,9 +91,10 @@ def plan_windows(frame_off: np.ndarray, h: int, max_window_points: int) -> np.nd
 
 def stdbscan_windowed(x: torch.Tensor, y: Optional[torch.Tensor], z: Optional[torch.Tensor], frame_off: np.ndarray,
                       frame_ids: np.ndarray, cuts: np.ndarray, eps_space: float, eps_time: float, min_samples: int,
-                      bounds4: Optional[np.ndarray] = None):
+                      bounds4: Optional[np.ndarray] = None, min_frames: Optional[int] = None):
     """``rb_stdbscan_windowed`` on SoA device tensors: returns ``(labels int32, core uint8, n_clusters)``. ``bounds4`` =
-    a box ``[x_min, x_max, y_min, y_max]`` containing every 2-D point: the plans then do not sync."""
+    a box ``[x_min, x_max, y_min, y_max]`` containing every 2-D point: the plans then do not sync. ``min_frames`` set:
+    ``rb_stdbscan_windowed_wf``, the PointCloudWorkF variant (``rb_stdbscan_wf``'s labels and core flags)."""
     ctx = context(x.device.index)
     off = np.ascontiguousarray(frame_off, dtype=np.int64)
     ids = np.ascontiguousarray(frame_ids, dtype=np.float32)
@@ -106,10 +108,15 @@ def stdbscan_windowed(x: torch.Tensor, y: Optional[torch.Tensor], z: Optional[to
         hint.lo[0], hint.hi[0], hint.lo[1], hint.hi[1] = (float(v) for v in bounds4)
         hint.times_integer = 1
     ncl = C.c_int64(0)
-    check(ctx.lib.rb_stdbscan_windowed(ctx.handle, ptr(x), ptr(y), ptr(z), 1, off.ctypes.data, ids.ctypes.data, len(ids), cu.ctypes.data,
-                                       len(cu) - 1, float(eps_space), float(np.float32(eps_time)), int(min_samples),
-                                       C.byref(hint) if hint is not None else None, ptr(labels), ptr(core), C.byref(ncl), stream_ptr()),
-          "rb_stdbscan_windowed")
+    common = (ctx.handle, ptr(x), ptr(y), ptr(z), 1, off.ctypes.data, ids.ctypes.data, len(ids), cu.ctypes.data, len(cu) - 1,
+              float(eps_space), float(np.float32(eps_time)), int(min_samples))
+    tail = (C.byref(hint) if hint is not None else None, ptr(labels), ptr(core), C.byref(ncl), stream_ptr())
+    if min_frames is None:
+        check(ctx.lib.rb_stdbscan_windowed(*common, *tail), "rb_stdbscan_windowed")
+    else:
+        if isinstance(min_frames, bool) or not isinstance(min_frames, (int, np.integer)):
+            raise RadarB200Error(f"min_frames must be None or an int >= 1, not {min_frames!r}")
+        check(ctx.lib.rb_stdbscan_windowed_wf(*common, int(min_frames), *tail), "rb_stdbscan_windowed_wf")
     return labels[:n], core[:n], int(ncl.value)
 
 
@@ -123,7 +130,8 @@ class RecordingResult(DetectionResult):
     """Device-resident result of a whole recording: the fields of :class:`DetectionResult` (its ``to_host``,
     ``to_frames``, ``clusters_by_frame`` and ``clusters_by_frame_host`` apply unchanged - the cluster records are built
     over frame chunks small enough for the records' slot table), plus the clustering's window cuts and what ran."""
-    core: Optional[torch.Tensor] = None                 # uint8 [points.n]: core flags of the clustered points
+    core: Optional[torch.Tensor] = None                 # uint8 [points.n]: core flags of the clustered points (with
+                                                        # config.min_frames: the PointCloudWorkF variant's)
     cuts: Optional[np.ndarray] = None                   # window cuts (frame indices) of the clustering
     frames_built: int = 0
     land_ordered: bool = False                          # non-integer intensities: the ordered accumulation ran
@@ -425,7 +433,7 @@ class RecordingDetection:
             cuts = plan_windows(p_off, h_t, self.window_budget(pts.n))
             z = pts.inten if cfg.cluster_3d else None
             labels, core, n_clusters = stdbscan_windowed(pts.x, pts.y, z, p_off, ids, cuts, cfg.eps_space, cfg.eps_time,
-                                                         cfg.min_samples, bounds4=self._b4)
+                                                         cfg.min_samples, bounds4=self._b4, min_frames=cfg.min_frames)
         timings["cluster"] = time.perf_counter() - t0
         return RecordingResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum, core=core, cuts=cuts,
                                frames_built=built, land_ordered=land_ordered, timings=timings,

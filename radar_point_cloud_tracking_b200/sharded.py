@@ -472,6 +472,8 @@ class ShardedDetection:
         from .pipeline import DetectionConfig
 
         self.cfg = config or DetectionConfig()
+        if self.cfg.min_frames is not None:
+            raise RadarB200Error("ShardedDetection does not run the min_frames variant: use RecordingDetection on one GPU")
         self.group = group
         self.rank = dist.get_rank(group) if rank is None else rank
         self.world = dist.get_world_size(group) if world is None else world
