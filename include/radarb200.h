@@ -108,14 +108,35 @@ int rb_expand_frame_times(rb_ctx* ctx, const int64_t* frame_off, const float* fr
 /* ---- a3: max fusion on a grid (T5:222-273 fuse_gains_max) --------------------------------------
  * Pools n points on a grid anchored at (x_min, y_min): cell = trunc((v - v_min)/res) in float32
  * (T5:258-259), keeps the max intensity per cell (T5:263) and emits occupied cells in y-major
- * order (T5:267): cell_ix, cell_iy int32 and max intensity float32, capacity cap_cells. The cell
- * centres x_min + ix*res + res/2 are float64 host arithmetic (T5:269-270) and stay in Python.
- * x_min / y_min / nx / ny are the host's float32 numpy values (T5:251-256). n_cells_out: host
- * int64. Syncs. */
+ * order (T5:267): cell_ix, cell_iy int32 and max intensity float32, capacity cap_cells.
+ * x_min / y_min / nx / ny are the caller's float32 values (T5:251-256). n_cells_out: host
+ * int64. Runs on the kernels of rb_fuse_max_frames (one frame, the caller's grid). Syncs. */
 int rb_fuse_max(rb_ctx* ctx, const float* x, const float* y, const float* inten, int64_t n,
                 float x_min, float y_min, float resolution, int nx, int ny,
                 int32_t* cell_ix, int32_t* cell_iy, float* cell_max, int64_t cap_cells,
                 int64_t* n_cells_out, void* stream);
+
+/* Max fusion of many frames per call: for every frame f (points [frame_off[f], frame_off[f+1]) of x, y, inten; frame_off
+ * int64[F+1] device, from 0 to n), exactly what fuse_gains_max returns for that frame's points:
+ *   bounds = the float32 min / max of the frame's points, nx = int(ceil((x_max - x_min) / res)) + 1 and likewise ny, and
+ *   cell = trunc((v - v_min) / res), all in float32 with res = (float)resolution (numpy >= 2, T5:251-259); max intensity
+ *   per cell starting from 0 (T5:262-263); cells > 0 in y-major order (T5:267) with float64 centres
+ *   x_min + ix * resolution + resolution / 2 evaluated left to right with the full double resolution (T5:269-270).
+ * Outputs (device): cell_x, cell_y float64 and cell_max float32 with capacity cap_cells (n always suffices: a frame has at
+ * most one cell per point); cell_off int64[F+1] delimits the frames. n_cells_out: host int64, the total.
+ * A frame's grid must have fewer than 2^30 cells (RB_ERR_ARG naming the frame otherwise). Frames are pooled in groups of
+ * consecutive frames whose grids fit a scratch bound together (2^28 cells, rb_set_option "fuse_group_cells"; a larger
+ * frame is a group alone). RB_ERR_ARG before anything is enqueued for a resolution that is not finite and > 0, F < 0,
+ * or NULL pointers. Syncs twice, whatever F: grid sizes, then the total. */
+int rb_fuse_max_frames(rb_ctx* ctx, const float* x, const float* y, const float* inten, int64_t n,
+                       const int64_t* frame_off, int64_t n_frames, double resolution,
+                       double* cell_x, double* cell_y, float* cell_max, int64_t cap_cells,
+                       int64_t* cell_off, int64_t* n_cells_out, void* stream);
+
+/* HOST function: rb_fuse_max_frames' grouping. cells[F] = grid cells of each frame; consecutive frames join a group while
+ * their cells add up to at most max_cells (a frame above it is a group alone). Writes the group cuts (frame indices,
+ * cuts[0] = 0 ... cuts[K] = F; at most cap entries) and returns K, or a negative RB_ERR_* for bad arguments. */
+int64_t rb_fuse_plan_groups(const int64_t* cells, int64_t n_frames, int64_t max_cells, int64_t* cuts, int64_t cap);
 
 /* ---- a4-a6: land / stationary persistence filter --------------------------------------------- */
 /* Global bounds (T4:365-369): out4 = device float32 {x_min, x_max, y_min, y_max}. No sync. */

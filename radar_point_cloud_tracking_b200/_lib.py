@@ -71,6 +71,9 @@ SIGNATURES = {
     "rb_expand_frame_times": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp]),
     "rb_fuse_max": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_i32, c_i32,
                             c_vp, c_vp, c_vp, c_i64, C.POINTER(c_i64), c_vp]),
+    "rb_fuse_max_frames": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_f64, c_vp, c_vp, c_vp, c_i64, c_vp,
+                                   C.POINTER(c_i64), c_vp]),
+    "rb_fuse_plan_groups": (c_i64, [c_vp, c_i64, c_i64, c_vp, c_i64]),
     "rb_bounds": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "rb_bounds_counted": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "rb_land_accumulate": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp]),

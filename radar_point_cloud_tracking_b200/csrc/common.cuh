@@ -39,7 +39,9 @@ enum rb_slot {
     RB_S_SLABEL,
     RB_S_STATS,
     RB_S_MISC,
-    RB_S_FUSE_GRID,
+    RB_S_FUSE_GRID,         // max fusion: the dense grids of one group of frames
+    RB_S_FUSE_FRAMES,       // max fusion: per-frame bounds, grid sizes and offsets
+    RB_S_FUSE_TILES,        // max fusion: occupied cells per grid tile, their scan
     RB_S_COMP_KEY,          // dbscan: component key per point (original order)
     RB_S_PIPE, RB_S_PIPE_EDGES, RB_S_PIPE_TIMES,   // rb_detect_block: sweep bases + bounds, device edges, times
     RB_S_B_NCORE, RB_S_B_PARENT, RB_S_B_LABEL, RB_S_B_MINKEY, RB_S_CORE_START, RB_S_CB_LIST,   // dbscan, tight: per-bucket arrays
@@ -84,6 +86,7 @@ struct rb_ctx {
     int opt_mask_priority = 1;       // 1: the mask kernel is launched with the device's highest launch priority
     int prio_high = 0;               // that priority (cudaDeviceGetStreamPriorityRange)
     int opt_mask_gate = 1;           // 1: the mask kernels of all contexts of a device run one after the other (see spoke.cu)
+    int64_t opt_fuse_group_cells = 0; // > 0: grid cells one group of rb_fuse_max_frames may hold (0 = 2^28)
     int opt_carveout = -1;           // >= 0: every launch asks for this shared-memory carve-out (percent), see rb_launch
     unsigned attr_spoke_mask = 0;    // per-context "function attribute set" flags (a context = one device)
     bool attr_land = false;

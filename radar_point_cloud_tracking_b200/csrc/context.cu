@@ -119,6 +119,11 @@ extern "C" int rb_set_option(rb_ctx* ctx, const char* name, int64_t value) {
         ctx->opt_carveout = (int)value;
         return RB_OK;
     }
+    if (!strcmp(name, "fuse_group_cells")) {
+        RB_REQUIRE(value >= 0, "fuse_group_cells: 0 = default (2^28), else the grid cells one group of frames may hold");
+        ctx->opt_fuse_group_cells = value;
+        return RB_OK;
+    }
     rb_set_error("rb_set_option: unknown option '%s'", name);
     return RB_ERR_ARG;
 }
@@ -135,6 +140,7 @@ extern "C" int64_t rb_get_info(rb_ctx* ctx, const char* name) {
     if (!strcmp(name, "mask_gate")) return ctx->opt_mask_gate;
     if (!strcmp(name, "mask_priority")) return ctx->opt_mask_priority;
     if (!strcmp(name, "carveout")) return ctx->opt_carveout;
+    if (!strcmp(name, "fuse_group_cells")) return ctx->opt_fuse_group_cells;
     // device time of the last profiled rb_spoke_to_points, per kernel, in nanoseconds (syncs on its last event)
     int k = !strcmp(name, "spoke_mask_ns") ? 0 : !strcmp(name, "spoke_offsets_ns") ? 1 : !strcmp(name, "spoke_emit_ns") ? 2 : -1;
     if (k >= 0) {

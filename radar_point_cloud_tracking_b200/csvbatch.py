@@ -147,6 +147,58 @@ def parse_files(paths: Sequence[Path], num_echo_columns: int, device=None) -> Li
     return resolve_batch(parsed, hn, [(Path(p), int(o), len(r)) for p, o, r in zip(paths, offs, raws)], num_echo_columns)
 
 
+def spoke_batch(results: Sequence[Sequence[Tuple[int, FileResult]]], E: int, angle_scale: float, device: torch.device,
+                append: Callable, timings: Dict[str, float], files: Optional[Dict[str, int]] = None) -> np.ndarray:
+    """Spoke stage of one batch of parsed frames (``results`` as :meth:`SweepReader.run` hands them out): per frame the
+    sweeps in order, each labelled with its gain key; files without a sweep add nothing. Frames whose host-parsed echoes
+    are all 0..255 integers travel as uint8 (``rb_spoke_to_points_u8``), others as float32. Runs of consecutive sweeps of
+    the same spoke count and echo type go to ``append(echo[W,S,E], cos, sin, range_res, sweep_gain)`` one launch each, in
+    sweep order; it returns the host point offsets ``[W+1]`` of the run's sweeps from the run's first point. Returns the
+    frames' point offsets ``[F+1]`` from the batch's first point. ``files`` counts the "batched" and "per_file" files;
+    ``timings`` gains "lead" (leading fields, trig tables) and "spoke"."""
+    from .tracker import sweep_tables
+
+    t0 = time.perf_counter()
+    sweeps, per_frame = [], []                           # sweeps: (gain label, angle, scale, echo device tensor, batch rows)
+    for frame in results:
+        for _, r in frame:
+            if files is not None:
+                files["per_file" if r.status is None else "batched"] += 1
+        got = [(g, r.sweep, r.rows) for g, r in frame if r.sweep is not None and r.sweep[2].shape[0] > 0]
+        host = [isinstance(sw[2], np.ndarray) for _, sw, _ in got]
+        as_u8 = [sw[2].astype(np.uint8) if h else None for (_, sw, _), h in zip(got, host)]
+        exact = all(np.array_equal(u, sw[2]) for (_, sw, _), u, h in zip(got, as_u8, host) if h)
+        for (g, sw, rows), u, h in zip(got, as_u8, host):
+            if exact:                                    # 0..255 integers travel as uint8 (rb_spoke_to_points_u8)
+                echo = torch.from_numpy(u).to(device) if h else sw[2]
+            else:                                        # the frame goes through the float32 kernel
+                echo = torch.from_numpy(np.ascontiguousarray(sw[2], np.float32)).to(device) if h else sw[2].float()
+                rows = None
+            sweeps.append((g, sw[0], sw[1], echo, None if h else rows))
+        per_frame.append(len(got))
+    tl = time.perf_counter()
+    timings["lead"] = timings.get("lead", 0.0) + tl - t0
+    sweep_off = [np.zeros(1, np.int64)]
+    for a, b in sweep_runs([(sw[3].shape[0], sw[3].dtype) for sw in sweeps]):
+        run = sweeps[a:b]
+        S = run[0][3].shape[0]
+        rows = [sw[4] for sw in run]
+        if all(r is not None for r in rows) and all(rows[i][1] == rows[i + 1][0] for i in range(len(rows) - 1)):
+            # consecutive rows of the batch's echo (same storage): a view, no copy
+            echo = run[0][3].as_strided((b - a, S, E), (S * E, E, 1))
+        else:
+            echo = torch.stack([sw[3] for sw in run])
+        t1 = time.perf_counter()
+        c, s_, r = sweep_tables(np.stack([sw[1] for sw in run]), np.stack([sw[2] for sw in run]), E, angle_scale)
+        timings["lead"] += time.perf_counter() - t1
+        gains = torch.tensor([sw[0] for sw in run], dtype=torch.int32, device=device)
+        off = append(echo, *(torch.from_numpy(np.ascontiguousarray(t)).to(device) for t in (c, s_, r)), gains)
+        sweep_off.append(off[1:] + sweep_off[-1][-1])
+    out = frame_offsets(np.concatenate(sweep_off), per_frame)
+    timings["spoke"] = timings.get("spoke", 0.0) + time.perf_counter() - tl
+    return out
+
+
 # ---- the reader ------------------------------------------------------------------------------------------------------
 def _read_into(buf: np.ndarray, path: Path, size: int) -> bool:
     """``size`` bytes of ``path`` into ``buf``; False when the file cannot be read or no longer has that size."""

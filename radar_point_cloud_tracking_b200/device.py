@@ -234,6 +234,53 @@ def fuse_max_cells(x: torch.Tensor, y: torch.Tensor, inten: torch.Tensor, x_min:
     return ix[:k], iy[:k], mx[:k]
 
 
+def check_resolution(resolution) -> float:
+    """``resolution`` as a float if it is finite and > 0; raises :class:`RadarB200Error` otherwise (no device work)."""
+    try:
+        r = float(resolution)
+    except (TypeError, ValueError):
+        raise RadarB200Error(f"grid_resolution must be a finite number > 0, not {resolution!r}") from None
+    if not (np.isfinite(r) and r > 0):
+        raise RadarB200Error(f"grid_resolution must be a finite number > 0, not {resolution!r}")
+    return r
+
+
+def fuse_max_frames(batch: PointBatch, resolution: float):
+    """``rb_fuse_max_frames`` over the frames of ``batch``: ``(cell_x f64, cell_y f64, cell_max f32, cell_off int64[F+1])``
+    on the device, frame f's cells being ``[cell_off[f], cell_off[f+1])``. Two syncs, whatever the number of frames."""
+    res = check_resolution(resolution)
+    ctx = context(batch.x.device.index)
+    d = batch.x.device
+    n = int(batch.n)
+    F = batch.frame_off.numel() - 1
+    if F < 0:
+        raise RadarB200Error("frame_off needs at least one entry")
+    x, y, inten = (_dev(t[:n], torch.float32, k) for t, k in ((batch.x, "x"), (batch.y, "y"), (batch.inten, "inten")))
+    off = _dev(batch.frame_off, torch.int64, "frame_off")
+    cx = torch.empty(max(n, 1), dtype=torch.float64, device=d)
+    cy = torch.empty(max(n, 1), dtype=torch.float64, device=d)
+    cm = torch.empty(max(n, 1), dtype=torch.float32, device=d)
+    cell_off = torch.empty(F + 1, dtype=torch.int64, device=d)
+    total = C.c_int64(0)
+    check(ctx.lib.rb_fuse_max_frames(ctx.handle, ptr(x), ptr(y), ptr(inten), n, ptr(off), F, res, ptr(cx), ptr(cy), ptr(cm), n,
+                                     ptr(cell_off), C.byref(total), stream_ptr()), "rb_fuse_max_frames")
+    k = total.value
+    return cx[:k], cy[:k], cm[:k], cell_off
+
+
+def fuse_plan_groups(cells, max_cells: int) -> np.ndarray:
+    """``rb_fuse_plan_groups`` (host): group cuts of frames with ``cells[f]`` grid cells under a bound of ``max_cells``."""
+    lib = _lib.load()
+    c = np.ascontiguousarray(cells, dtype=np.int64)
+    k = int(lib.rb_fuse_plan_groups(c.ctypes.data, len(c), int(max_cells), None, 0))
+    if k < 0:
+        check(k, "rb_fuse_plan_groups")
+    cuts = np.zeros(k + 1, dtype=np.int64)
+    check(0 if lib.rb_fuse_plan_groups(c.ctypes.data, len(c), int(max_cells), cuts.ctypes.data, k + 1) == k else -2,
+          "rb_fuse_plan_groups")
+    return cuts
+
+
 # --------------------------------------------------------------------------------------- a4-a6
 def bounds(x: torch.Tensor, y: torch.Tensor) -> torch.Tensor:
     """Device float32 ``[x_min, x_max, y_min, y_max]`` (no sync)."""

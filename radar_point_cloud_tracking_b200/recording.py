@@ -306,48 +306,12 @@ class RecordingDetection:
     def _add_csv_batch(self, results, ids: np.ndarray, times: list, E: int) -> None:
         """Spoke stage of one batch of parsed frames (see :meth:`add_csv_frames`), booked as one block."""
         from . import csvbatch
-        from .tracker import sweep_tables
 
-        t0 = time.perf_counter()
-        d, cfg = self.device, self.cfg
-        sweeps, per_frame = [], []                       # sweeps: (gain label, angle, scale, echo device tensor, batch rows)
-        for frame in results:
-            for _, r in frame:
-                self.csv_files["per_file" if r.status is None else "batched"] += 1
-            got = [(g, r.sweep, r.rows) for g, r in frame if r.sweep is not None and r.sweep[2].shape[0] > 0]
-            host = [isinstance(sw[2], np.ndarray) for _, sw, _ in got]
-            as_u8 = [sw[2].astype(np.uint8) if h else None for (_, sw, _), h in zip(got, host)]
-            exact = all(np.array_equal(u, sw[2]) for (_, sw, _), u, h in zip(got, as_u8, host) if h)
-            for (g, sw, rows), u, h in zip(got, as_u8, host):
-                if exact:                                # 0..255 integers travel as uint8 (rb_spoke_to_points_u8)
-                    echo = torch.from_numpy(u).to(d) if h else sw[2]
-                else:                                    # the frame goes through the float32 kernel
-                    echo = torch.from_numpy(np.ascontiguousarray(sw[2], np.float32)).to(d) if h else sw[2].float()
-                    rows = None
-                sweeps.append((g, sw[0], sw[1], echo, None if h else rows))
-            per_frame.append(len(got))
-        tl = time.perf_counter()
-        self.timings["lead"] += tl - t0
         base = self._n
-        sweep_off = [np.zeros(1, np.int64)]
-        for a, b in csvbatch.sweep_runs([(sw[3].shape[0], sw[3].dtype) for sw in sweeps]):
-            run = sweeps[a:b]
-            S = run[0][3].shape[0]
-            rows = [sw[4] for sw in run]
-            if all(r is not None for r in rows) and all(rows[i][1] == rows[i + 1][0] for i in range(len(rows) - 1)):
-                # consecutive rows of the batch's echo (same storage): a view, no copy
-                echo = run[0][3].as_strided((b - a, S, E), (S * E, E, 1))
-            else:
-                echo = torch.stack([sw[3] for sw in run])
-            t1 = time.perf_counter()
-            c, s_, r = sweep_tables(np.stack([sw[1] for sw in run]), np.stack([sw[2] for sw in run]), E, cfg.angle_scale)
-            self.timings["lead"] += time.perf_counter() - t1
-            gains = torch.tensor([sw[0] for sw in run], dtype=torch.int32, device=d)
-            off = self._spoke_append(echo, *(torch.from_numpy(np.ascontiguousarray(t)).to(d) for t in (c, s_, r)), gains,
-                                     lambda sweep_base: sweep_base)
-            sweep_off.append(off[1:] + sweep_off[-1][-1])
-        self._add_frames(base, csvbatch.frame_offsets(np.concatenate(sweep_off), per_frame), ids, times)
-        self.timings["spoke"] += time.perf_counter() - tl
+        off = csvbatch.spoke_batch(results, E, self.cfg.angle_scale, self.device,
+                                   lambda echo, c, s, r, gains: self._spoke_append(echo, c, s, r, gains, lambda sweep_base: sweep_base),
+                                   self.timings, self.csv_files)
+        self._add_frames(base, off, ids, times)
 
     # ---- the recording ------------------------------------------------------------------------------------------------
     def window_budget(self, n_points: int) -> int:
