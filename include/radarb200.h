@@ -514,6 +514,30 @@ int rb_csv_parse_sweeps(rb_ctx* ctx, const uint8_t* text, int64_t n_bytes, const
  * All pointers are host pointers. The header is the caller's business. */
 int rb_ply_append_ascii(const char* path, const float* x, const float* y, const float* z, const uint8_t* rgb, int64_t n);
 
+/* The same vertex lines formatted on the device, for every float32 value (no printf): the lines of x, y, z float32[n]
+ * and rgb uint8[n][3], concatenated into text (capacity cap bytes), and line_end int64[n] = the end offset of every line
+ * in text. total: device int64[1] = the bytes of all lines. When total > cap nothing is written to text (line_end and
+ * total still are): the caller reads total back and calls again with a larger buffer. Three launches, no sync. */
+int rb_ply_format_ascii(rb_ctx* ctx, const float* x, const float* y, const float* z, const uint8_t* rgb, int64_t n,
+                        char* text, int64_t cap, int64_t* line_end, int64_t* total, void* stream);
+
+/* The 15-byte little-endian records of write_ply_binary (WF:797-827): out[15 * i ..] = x, y, z float32 then r, g, b.
+ * One launch, no sync. */
+int rb_ply_pack_binary(rb_ctx* ctx, const float* x, const float* y, const float* z, const uint8_t* rgb, int64_t n,
+                       uint8_t* out, void* stream);
+
+/* intensity_to_rgb (T5:292-327) of values[n], float32 (is_f64 = 0) or float64 (is_f64 = 1), with numpy >= 2's dtype rules
+ * (all arithmetic in the input's dtype, ramps truncated to uint8), into rgb uint8[n][3]. normalize = 1 first applies
+ * normalize_intensity (T5:276-289) to each frame [frame_off[f], frame_off[f+1]) of frame_off int64[n_frames + 1] (numpy's
+ * linear 99th percentile and the minimum of the frame; elements outside every frame are not written). A NaN or a value
+ * outside [0, 255] after the optional normalisation has no defined colour in the reference: it sets bit 0 of status
+ * (device int32[1], cleared by the call) and is coloured black. One launch (normalize: one block per frame), no sync. */
+int rb_ply_colors_intensity(rb_ctx* ctx, const void* values, int is_f64, int64_t n, const int64_t* frame_off,
+                            int64_t n_frames, int normalize, uint8_t* rgb, int32_t* status, void* stream);
+
+/* gain_to_rgb (T5:330-342): the GAIN_COLORS colour of each int32 gain, black for any other gain. One launch, no sync. */
+int rb_ply_colors_gain(rb_ctx* ctx, const int32_t* gains, int64_t n, uint8_t* rgb, void* stream);
+
 /* ---- test/bench infrastructure (not part of the reference surface) ---------------------------
  * Device twin of radar_point_cloud_tracking_b200.synthetic.synth_echo: fills echo[W][S][E] for
  * sweeps w0 .. w0+n_sweeps-1 of the data set. sweep_keys uint32[n_sweeps], clutter_thr

@@ -123,6 +123,10 @@ SIGNATURES = {
     "rb_csv_parse_sweeps": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i32, c_i32, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp,
                                     c_vp, c_vp, c_vp]),
     "rb_ply_append_ascii": (c_i32, [C.c_char_p, c_vp, c_vp, c_vp, c_vp, c_i64]),
+    "rb_ply_format_ascii": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "rb_ply_pack_binary": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
+    "rb_ply_colors_intensity": (c_i32, [c_vp, c_vp, c_i32, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp]),
+    "rb_ply_colors_gain": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp]),
     "rb_synth_echo": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_i32, c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "rb_set_option": (c_i32, [c_vp, C.c_char_p, c_i64]),
     "rb_get_info": (c_i64, [c_vp, C.c_char_p]),

@@ -57,6 +57,7 @@ enum rb_slot {
     RB_S_REC_KEYS_BIG,      // windowed ST-DBSCAN: encodings of the windows that outgrew the capacity guess
     RB_S_REC_TABLE,         // windowed ST-DBSCAN: the stitched key -> cluster id table
     RB_S_REC_CORE,          // windowed ST-DBSCAN: recording-wide core flags when the caller passes none
+    RB_S_PLY_TILES,         // PLY formatter: bytes of each block of lines, then their scan
     RB_S_COUNT
 };
 

@@ -170,7 +170,8 @@ class _BatchPoints:
 
 
 def fuse_csv_frames_max(frame_files: Sequence[Mapping[int, "os.PathLike"]], grid_resolution: float = 1.0, batch_bytes: int = 64 << 20,
-                        readers: Optional[int] = None, _cfg=None, timings: Optional[Dict[str, float]] = None) -> List[Points]:
+                        readers: Optional[int] = None, _cfg=None, timings: Optional[Dict[str, float]] = None,
+                        ply_paths: Optional[Sequence["os.PathLike"]] = None) -> List[Points]:
     """``fuse_gains_max(frame_files[f], grid_resolution)`` for every frame of a recording: one ``(x, y, max_intensity)`` per
     frame, equal to the reference's with the configuration globals ``NUM_ECHO_COLUMNS``, ``INTENSITY_THRESHOLD`` and
     ``POINT_STRIDE`` (``_cfg`` = :func:`_config` of a T5 module; default this module's). File handling is that of
@@ -178,7 +179,10 @@ def fuse_csv_frames_max(frame_files: Sequence[Mapping[int, "os.PathLike"]], grid
     whole frames (at most ``batch_bytes``) per ``rb_csv_parse_sweeps`` launch; unreadable files print the reference's
     message and add no points, as do empty and header-only ones; files outside the device grammar or larger than a batch
     take the per-file readers. Each batch is fused as it arrives (spoke stage, then :func:`fuse_frames_max`), so device
-    memory follows one batch, not the recording. ``timings`` (optional) accumulates the seconds of each stage."""
+    memory follows one batch, not the recording. ``timings`` (optional) accumulates the seconds of each stage.
+    ``ply_paths`` (optional, one path per frame): each batch's fused frames are also written from the device as the batch
+    arrives, file f with the bytes of ``write_ply_fast(ply_paths[f], x, y, max_intensity, intensity_to_rgb(max_intensity))``
+    and its ``Wrote`` line (``plyio.intensity_rgb`` and ``plyio.write_ply_frames``, stage "ply")."""
     from . import csvbatch
 
     res = dev.check_resolution(grid_resolution)
@@ -189,6 +193,10 @@ def fuse_csv_frames_max(frame_files: Sequence[Mapping[int, "os.PathLike"]], grid
     if not (csvbatch.CSV_CHUNK <= int(batch_bytes) <= csvbatch.MAX_BATCH_BYTES):
         raise RadarB200Error(f"batch_bytes must be in [{csvbatch.CSV_CHUNK}, {csvbatch.MAX_BATCH_BYTES}]")
     frames = [sorted((g, Path(p)) for g, p in ff.items()) for ff in frame_files]
+    if ply_paths is not None:
+        ply_paths = [Path(p) for p in ply_paths]
+        if len(ply_paths) != len(frames):
+            raise RadarB200Error(f"{len(ply_paths)} PLY paths for {len(frames)} frames")
     if not frames:
         return []
     if not torch.cuda.is_available():
@@ -197,7 +205,7 @@ def fuse_csv_frames_max(frame_files: Sequence[Mapping[int, "os.PathLike"]], grid
 
     d = torch.device("cuda", torch.cuda.current_device())
     timings = {} if timings is None else timings
-    for k in ("read", "h2d", "parse", "lead", "spoke", "fuse"):
+    for k in ("read", "h2d", "parse", "lead", "spoke", "fuse") + (("ply",) if ply_paths is not None else ()):
         timings.setdefault(k, 0.0)
     pts = _BatchPoints(d, cfg.INTENSITY_THRESHOLD, cfg.POINT_STRIDE)
     out: List[Points] = []
@@ -206,8 +214,16 @@ def fuse_csv_frames_max(frame_files: Sequence[Mapping[int, "os.PathLike"]], grid
         pts.reset()
         off = csvbatch.spoke_batch(results, E, ANGLE_SCALE, d, pts.append, timings)
         t0 = time.perf_counter()
-        out.extend(fuse_frames_max(pts.batch(off), res).frames())
+        fused = fuse_frames_max(pts.batch(off), res)
+        out.extend(fused.frames())
         timings["fuse"] += time.perf_counter() - t0
+        if ply_paths is not None:
+            from . import plyio
+
+            t0 = time.perf_counter()
+            plyio.write_ply_frames(ply_paths[fa:fb], fused.cell_x, fused.cell_y, fused.cell_max, plyio.intensity_rgb(fused.cell_max),
+                                   fused.cell_off)
+            timings["ply"] += time.perf_counter() - t0
 
     csvbatch.SweepReader().run(frames, E, d, readers or min(8, os.cpu_count() or 1), consume, timings, batch_bytes)
     return out

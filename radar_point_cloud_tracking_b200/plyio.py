@@ -5,15 +5,20 @@ arguments and bytes on disk.
   the body is written by the library's host function ``rb_ply_append_ascii`` (exact ``%.4f``, see ``csrc/plyfmt.cu``)
   instead of a float64 table formatted row by row in Python;
 * :func:`write_ply_binary` — the binary branch of ``PointCloudWorkF/stdbscan_denoising_pipeline.py:797-827``;
-* :func:`normalize_intensity`, :func:`intensity_to_rgb`, :func:`gain_to_rgb` — ``T5:276-342``.
+* :func:`normalize_intensity`, :func:`intensity_to_rgb`, :func:`gain_to_rgb` — ``T5:276-342``;
+* whole recordings from the device: :func:`intensity_rgb` / :func:`gain_rgb` colour device tensors on the device, and
+  :func:`write_ply_frames` writes one file per frame with the bytes of :func:`write_ply_fast` (or
+  :func:`write_ply_binary`), formatted on the device many frames per launch.
 
 Coordinates / colours may be numpy arrays or torch tensors (device tensors are brought back once).
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
+import threading
 from pathlib import Path
-from typing import Dict, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -125,3 +130,243 @@ def write_ply_binary(path: Path, x, y, z, colors) -> None:
     with path.open("wb") as fh:
         fh.write(_HEADER.format(fmt="binary_little_endian", n=len(x)).encode("ascii"))
         rec.tofile(fh)
+
+
+# ---- whole recordings from the device -------------------------------------------------------------------------
+#: bytes of the longest vertex line "%.4f %.4f %.4f %d %d %d\n" (three 45-character floats); a chunk of text holds
+#: chunk_bytes // PLY_LINE_MAX lines, so it never overflows, whatever the values
+PLY_LINE_MAX = 150
+PLY_RECORD_BYTES = 15
+DEFAULT_CHUNK_BYTES = 256 << 20
+
+
+def _cuda(t, name: str):
+    import torch
+
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise _lib.RadarB200Error(f"{name} must be a CUDA tensor")
+    return t
+
+
+def _frame_offsets(frame_off, n: int, name: str = "frame_off") -> np.ndarray:
+    """Host copy of a device int64[F+1] offset tensor, checked: non-decreasing, within [0, n]."""
+    import torch
+
+    _cuda(frame_off, name)
+    if frame_off.dtype != torch.int64 or frame_off.dim() != 1 or frame_off.numel() < 1:
+        raise _lib.RadarB200Error(f"{name} must be a 1-D int64 tensor of F + 1 offsets")
+    off = frame_off.cpu().numpy()
+    if off[0] < 0 or off[-1] > n or np.any(np.diff(off) < 0):
+        raise _lib.RadarB200Error(f"{name} must be non-decreasing within [0, {n}]")
+    return off
+
+
+def intensity_rgb(values, frame_off=None, normalize: bool = False):
+    """``intensity_to_rgb`` of a float32 / float64 device tensor, on the device (uint8 ``[N, 3]`` CUDA tensor): each frame
+    ``[frame_off[f], frame_off[f+1])`` gets ``intensity_to_rgb(normalize_intensity(v))`` with ``normalize``, else
+    ``intensity_to_rgb(v)`` (without ``frame_off`` the whole tensor is one frame). Raises :class:`RadarB200Error` for a NaN
+    or a value outside [0, 255] after the optional normalisation: the reference's ``astype(np.uint8)`` has no defined
+    result there."""
+    import torch
+
+    _cuda(values, "values")
+    if values.dtype not in (torch.float32, torch.float64) or values.dim() != 1:
+        raise _lib.RadarB200Error("values must be a 1-D float32 or float64 tensor")
+    n = values.numel()
+    if frame_off is None:
+        frame_off = torch.tensor([0, n], dtype=torch.int64, device=values.device)
+    elif frame_off.device != values.device:
+        raise _lib.RadarB200Error("frame_off must be on the device of values")
+    off = _frame_offsets(frame_off, n)
+    ctx = _lib.context(values.device.index)
+    v = values.contiguous()
+    rgb = torch.zeros((n, 3), dtype=torch.uint8, device=values.device)
+    status = torch.empty(1, dtype=torch.int32, device=values.device)
+    with torch.cuda.device(values.device):
+        _lib.check(ctx.lib.rb_ply_colors_intensity(ctx.handle, _lib.ptr(v), int(v.dtype == torch.float64), n, _lib.ptr(frame_off),
+                                                   len(off) - 1, int(bool(normalize)), _lib.ptr(rgb), _lib.ptr(status),
+                                                   _lib.stream_ptr()), "rb_ply_colors_intensity")
+        if int(status.item()):
+            raise _lib.RadarB200Error("intensity_rgb: a value is NaN or outside [0, 255]" + (" after normalisation" if normalize else "")
+                                      + "; intensity_to_rgb has no defined colour for it")
+    return rgb
+
+
+def gain_rgb(gains):
+    """``gain_to_rgb`` of an int32 device tensor, on the device (uint8 ``[N, 3]`` CUDA tensor)."""
+    import torch
+
+    _cuda(gains, "gains")
+    if gains.dtype != torch.int32 or gains.dim() != 1:
+        raise _lib.RadarB200Error("gains must be a 1-D int32 tensor")
+    ctx = _lib.context(gains.device.index)
+    g = gains.contiguous()
+    rgb = torch.empty((g.numel(), 3), dtype=torch.uint8, device=g.device)
+    with torch.cuda.device(g.device):
+        _lib.check(ctx.lib.rb_ply_colors_gain(ctx.handle, _lib.ptr(g), g.numel(), _lib.ptr(rgb), _lib.stream_ptr()),
+                   "rb_ply_colors_gain")
+    return rgb
+
+
+def plan_chunks(off: np.ndarray, lines_per_chunk: int):
+    """Cut the vertices ``[off[0], off[-1])`` into chunks of at most ``lines_per_chunk`` lines. Returns a list of
+    ``(v0, v1, pieces)``: ``pieces`` = ``(frame, a, b)`` vertex ranges of the chunk in frame order. A frame spanning chunks
+    has a piece in each; a frame without vertices has one empty piece, in the chunk that holds its position (the last
+    chunk for the end), so every frame's last piece comes no earlier than the previous frame's."""
+    if lines_per_chunk < 1:
+        raise _lib.RadarB200Error("a chunk must hold at least one line")
+    start, end = int(off[0]), int(off[-1])
+    n_chunks = max(1, -(-(end - start) // lines_per_chunk))
+    bounds = [(start + k * lines_per_chunk, min(end, start + (k + 1) * lines_per_chunk)) for k in range(n_chunks)]
+    pieces = [[] for _ in range(n_chunks)]
+    for f in range(len(off) - 1):
+        a, b = int(off[f]), int(off[f + 1])
+        if a == b:
+            pieces[min((a - start) // lines_per_chunk, n_chunks - 1)].append((f, a, a))
+            continue
+        for k in range((a - start) // lines_per_chunk, (b - 1 - start) // lines_per_chunk + 1):
+            v0, v1 = bounds[k]
+            pieces[k].append((f, max(a, v0), min(b, v1)))
+    return [(v0, v1, p) for (v0, v1), p in zip(bounds, pieces)]
+
+
+_ply_staging = threading.local()
+
+
+def _pinned_pair(nbytes: int):
+    """This thread's two pinned staging buffers of at least ``nbytes`` each, kept from call to call."""
+    import torch
+
+    bufs = getattr(_ply_staging, "bufs", None)
+    if bufs is None or bufs[0].numel() < nbytes:
+        _ply_staging.bufs = None
+        _ply_staging.bufs = bufs = [torch.empty(nbytes, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+    return bufs
+
+
+def _write_piece(path: Path, header: Optional[bytes], body) -> None:
+    try:
+        with path.open("wb" if header is not None else "ab") as fh:
+            if header is not None:
+                fh.write(header)
+            fh.write(body)
+    except OSError as e:
+        raise _lib.RadarB200Error(f"write_ply_frames: cannot write {path}: {e}") from None
+
+
+def write_ply_frames(paths: Sequence, x, y, z, colors, frame_off, binary: bool = False,
+                     chunk_bytes: int = DEFAULT_CHUNK_BYTES, writers: Optional[int] = None,
+                     timings: Optional[Dict[str, float]] = None) -> None:
+    """One PLY file per frame from device tensors: file k gets exactly the bytes of
+    ``write_ply_fast(paths[k], x[a:b], y[a:b], z[a:b], colors[a:b])`` (``write_ply_binary``'s with ``binary``) for
+    ``a, b = frame_off[k], frame_off[k+1]``, and in ASCII the same ``Wrote`` line is printed per file, in order.
+
+    ``x, y, z``: floating CUDA tensors (cast to float32 first), ``colors``: uint8 ``[N, 3]``, ``frame_off``: int64 ``[F+1]``
+    (``PointBatch.frame_off`` or ``FusedFrames.cell_off``), all on one device; ``len(paths) == F``. The text is formatted
+    on the device (``rb_ply_format_ascii`` / ``rb_ply_pack_binary``) in chunks of at most ``chunk_bytes``, never splitting a
+    line (a frame may span chunks: its file is appended in order), and copied into two pinned buffers that are kept from
+    call to call. While ``writers`` threads write one chunk's files, the next chunk is formatted and copied. A chunk costs
+    two syncs (one with ``binary``), whatever the number of frames in it. Every argument is checked before any device work
+    or file creation. ``timings`` (optional) accumulates the seconds of "format" (CUDA events), "d2h" and "write"."""
+    import time
+    from concurrent.futures import ThreadPoolExecutor
+
+    import torch
+
+    paths = [Path(p) for p in paths]
+    for name, t in (("x", x), ("y", y), ("z", z)):
+        _cuda(t, name)
+        if not t.is_floating_point() or t.dim() != 1:
+            raise _lib.RadarB200Error(f"{name} must be a 1-D floating tensor")
+    _cuda(colors, "colors")
+    if colors.dtype != torch.uint8 or colors.dim() != 2 or colors.shape[1] != 3:
+        raise _lib.RadarB200Error("colors must be a uint8 [N, 3] tensor")
+    _cuda(frame_off, "frame_off")
+    device = x.device
+    if any(t.device != device for t in (y, z, colors, frame_off)):
+        raise _lib.RadarB200Error("x, y, z, colors and frame_off must be on one device")
+    unit = PLY_RECORD_BYTES if binary else PLY_LINE_MAX
+    if int(chunk_bytes) < unit:
+        raise _lib.RadarB200Error(f"chunk_bytes must be at least {unit}")
+    n = min(x.numel(), y.numel(), z.numel(), colors.shape[0])
+    off = _frame_offsets(frame_off, n)
+    if len(paths) != len(off) - 1:
+        raise _lib.RadarB200Error(f"{len(paths)} paths for {len(off) - 1} frames")
+
+    timings = {} if timings is None else timings
+    for k in ("format", "d2h", "write"):
+        timings.setdefault(k, 0.0)
+    L = int(chunk_bytes) // unit
+    chunks = plan_chunks(off, L)
+    lines = max(v1 - v0 for v0, v1, _ in chunks)
+    ctx = _lib.context(device.index)
+    fmt = "binary_little_endian" if binary else "ascii"
+    last_piece = {f: (k, a, b) for k, (_, _, ps) in enumerate(chunks) for f, a, b in ps}
+    with torch.cuda.device(device):
+        xf, yf, zf = (t.to(torch.float32).contiguous() for t in (x, y, z))
+        rgb = colors.contiguous()
+        cap = max(lines * unit, 1)
+        text = torch.empty(cap, dtype=torch.uint8, device=device)
+        ends = torch.empty(max(lines, 1), dtype=torch.int64, device=device)
+        total = torch.empty(1, dtype=torch.int64, device=device)
+        ends_at = (cap + 7) & ~7
+        hosts = _pinned_pair(ends_at + 8 * max(lines, 1))
+        stream = torch.cuda.current_stream(device)
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+        pool = ThreadPoolExecutor(max_workers=writers or min(16, os.cpu_count() or 1))
+        pending: list = []
+        done: list = []
+
+        def finish_pending():
+            t0 = time.perf_counter()
+            for fut in pending:
+                fut.result()
+            timings["write"] += time.perf_counter() - t0
+            for f in done if not binary else ():               # write_ply_binary prints nothing
+                print(f"  Wrote {int(off[f + 1] - off[f]):,} points to {paths[f].name}")
+            pending.clear(), done.clear()
+
+        try:
+            for k, (v0, v1, pieces) in enumerate(chunks):
+                m = v1 - v0
+                host = hosts[k % 2]
+                ev[0].record(stream)
+                if binary:
+                    _lib.check(ctx.lib.rb_ply_pack_binary(ctx.handle, _lib.ptr(xf) + 4 * v0, _lib.ptr(yf) + 4 * v0, _lib.ptr(zf) + 4 * v0,
+                                                          _lib.ptr(rgb) + 3 * v0, m, _lib.ptr(text), _lib.stream_ptr()), "rb_ply_pack_binary")
+                else:
+                    _lib.check(ctx.lib.rb_ply_format_ascii(ctx.handle, _lib.ptr(xf) + 4 * v0, _lib.ptr(yf) + 4 * v0, _lib.ptr(zf) + 4 * v0,
+                                                           _lib.ptr(rgb) + 3 * v0, m, _lib.ptr(text), cap, _lib.ptr(ends),
+                                                           _lib.ptr(total), _lib.stream_ptr()), "rb_ply_format_ascii")
+                ev[1].record(stream)
+                t0 = time.perf_counter()
+                if binary:
+                    line_end = None
+                    nbytes = unit * m
+                else:
+                    line_end = host[ends_at:ends_at + 8 * max(m, 1)].view(torch.int64)
+                    if m:
+                        line_end[:m].copy_(ends[:m], non_blocking=True)
+                    stream.synchronize()
+                    nbytes = int(line_end[m - 1]) if m else 0
+                    line_end = line_end.numpy()
+                if nbytes:
+                    host[:nbytes].copy_(text[:nbytes], non_blocking=True)
+                stream.synchronize()
+                timings["d2h"] += time.perf_counter() - t0
+                timings["format"] += ev[0].elapsed_time(ev[1]) * 1e-3
+                finish_pending()                                  # the previous chunk's files, before this chunk appends
+                body = host.numpy()
+                for f, a, b in pieces:
+                    if binary:
+                        lo, hi = unit * (a - v0), unit * (b - v0)
+                    else:
+                        lo = int(line_end[a - v0 - 1]) if a > v0 else 0
+                        hi = int(line_end[b - v0 - 1]) if b > v0 else lo
+                    header = _HEADER.format(fmt=fmt, n=int(off[f + 1] - off[f])).encode("ascii") if a == off[f] else None
+                    pending.append(pool.submit(_write_piece, paths[f], header, memoryview(body[lo:hi])))
+                    if last_piece[f] == (k, a, b):
+                        done.append(f)
+            finish_pending()
+        finally:
+            pool.shutdown(wait=True, cancel_futures=True)
