@@ -554,7 +554,8 @@ int rb_synth_echo(rb_ctx* ctx, float* echo, int64_t n_sweeps, int n_spokes, int 
  * "dbscan_mode": 0 = auto (tight-cell bucket algorithm when the times are integers and the bucket table
  * fits the budget), 1 = always the general algorithm, 2 = require the tight one. */
 int rb_set_option(rb_ctx* ctx, const char* name, int64_t value);
-/* "launches"; "spoke_last_variant" (1 = register-staged, 2 = TMA-staged); "spoke_mask_ns" / "spoke_offsets_ns" / "spoke_emit_ns" = device time of the kernels of the
+/* "launches"; "spoke_last_variant" (1 = register-staged, 2 = TMA-staged); "land_last_variant" (accumulation kernel of the last
+ * rb_land_accumulate / rb_land_accumulate_ordered: 1 = shared-memory histogram, 2 = global atomics, 3 = ordered); "spoke_mask_ns" / "spoke_offsets_ns" / "spoke_emit_ns" = device time of the kernels of the
  * last profiled rb_spoke_to_points (syncs on its last event); -1 for unknown names or nothing recorded. */
 int64_t rb_get_info(rb_ctx* ctx, const char* name);
 

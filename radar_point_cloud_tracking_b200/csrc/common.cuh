@@ -81,6 +81,7 @@ struct rb_ctx {
     int opt_dbscan_mode = 0;         // 0 = auto, 1 = always the general algorithm, 2 = require the tight one
     int opt_spoke_mask_variant = 0;  // 0 = auto, 1 = register-staged mask kernel, 2 = require the TMA-staged one
     int spoke_last_variant = 0;      // mask kernel the last rb_spoke_to_points launched (1 / 2)
+    int land_last_variant = 0;       // accumulation the last rb_land_accumulate[_ordered] ran (1 = shared, 2 = global, 3 = ordered)
     int opt_spoke_profile = 0;       // 1: record events around the three spoke-to-point kernels
     int opt_spoke_ring = 2;          // TMA ring of the mask kernel: 0 = 64 KiB x 3, 1 = 32 KiB x 4, 2 = 32 KiB x 3 (default), 3 = 48 KiB x 2
     int opt_spoke_l2_hint = 1;       // 1: the mask kernel's bulk loads carry an L2 evict-first policy

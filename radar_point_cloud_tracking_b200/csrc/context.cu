@@ -135,6 +135,7 @@ extern "C" int64_t rb_get_info(rb_ctx* ctx, const char* name) {
     if (!strcmp(name, "spoke_mask_variant")) return ctx->opt_spoke_mask_variant;
     if (!strcmp(name, "dbscan_mode")) return ctx->opt_dbscan_mode;
     if (!strcmp(name, "spoke_last_variant")) return ctx->spoke_last_variant;
+    if (!strcmp(name, "land_last_variant")) return ctx->land_last_variant;
     if (!strcmp(name, "spoke_ring")) return ctx->opt_spoke_ring;
     if (!strcmp(name, "spoke_l2_hint")) return ctx->opt_spoke_l2_hint;
     if (!strcmp(name, "mask_gate")) return ctx->opt_mask_gate;

@@ -396,10 +396,12 @@ extern "C" int rb_land_accumulate(rb_ctx* ctx, const float* x, const float* y, c
             ctx->attr_land = true;
         }
         RB_CUDA(rb_launch(ctx, land_accumulate_smem, dim3(blocks), dim3(LD_THREADS), smem, stream, x, y, inten, n, g, count, isum, inexact));
+        ctx->land_last_variant = 1;
     } else {
         blocks = (int)(rb_div_up(n, LD_THREADS) < (int64_t)ctx->sm_count * 8 ? rb_div_up(n, LD_THREADS)
                                                                            : (int64_t)ctx->sm_count * 8);
         RB_CUDA(rb_launch(ctx, land_accumulate_global, dim3(blocks), dim3(LD_THREADS), 0, stream, x, y, inten, n, g, count, isum, inexact));
+        ctx->land_last_variant = 2;
     }
     RB_LAUNCH_CHECK(ctx);
     return RB_OK;
@@ -454,6 +456,7 @@ extern "C" int rb_land_accumulate_ordered(rb_ctx* ctx, const float* x, const flo
     const int blocks = (int)(rb_div_up(n, LD_THREADS) < (int64_t)ctx->sm_count * 8 ? rb_div_up(n, LD_THREADS) : (int64_t)ctx->sm_count * 8);
     RB_CUDA(rb_launch(ctx, land_cell_id_kernel, dim3(blocks), dim3(LD_THREADS), 0, stream, x, y, n, g, cell));
     RB_LAUNCH_CHECK(ctx);
+    ctx->land_last_variant = 3;
     int64_t n_seg = 0;
     RB_TRY(rb_stable_group(ctx, inten, cell, n, cells, seg_label, seg_count, seg_start, (int64_t)seg_cap, grouped, &n_seg, stream));
     if (n_seg > 0) {

@@ -60,10 +60,11 @@ def _run_sweeps(dev, echo_np, spec, thr, stride, gains=None, gpf=1, cap=None):
 
 # ------------------------------------------------------------------------------- synthetic twin
 def test_device_generator_matches_numpy(gpu):
-    spec = syn.SweepSpec(seed=9, frames=3, spokes=40, bins=256, clutter_p=0.02, land_blobs=2, buoys=3, boats=2)
-    assert np.array_equal(gpu.synth_echo(spec).cpu().numpy(), syn.synth_echo(spec))
-    part = gpu.synth_echo(spec, first_frame=1, n_frames=2).cpu().numpy()
-    assert np.array_equal(part, syn.synth_echo(spec)[1:])
+    for scale_m in (231.5, 2778.0):                 # boat positions depend on the range
+        spec = syn.SweepSpec(seed=9, frames=3, spokes=40, bins=256, clutter_p=0.02, land_blobs=2, buoys=3, boats=2, scale_m=scale_m)
+        assert np.array_equal(gpu.synth_echo(spec).cpu().numpy(), syn.synth_echo(spec))
+        part = gpu.synth_echo(spec, first_frame=1, n_frames=2).cpu().numpy()
+        assert np.array_equal(part, syn.synth_echo(spec)[1:])
 
 
 # ------------------------------------------------------------------------------- a1: spoke-to-point
