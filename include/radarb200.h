@@ -402,6 +402,43 @@ int rb_stdbscan_windowed_wf(rb_ctx* ctx, const float* x, const float* y, const f
                             int min_frames, const rb_stdbscan_hint* hint, int32_t* labels, uint8_t* core, int64_t* n_clusters,
                             void* stream);
 
+/* The three passes of rb_stdbscan_windowed(_wf) as entries of their own, over a LOCAL problem: frames [0, n_frames) of
+ * x/y/z with host frame offsets and ids as above, of which the windows (cuts_host[n_windows+1], from own_fa to own_fb)
+ * cover only the OWNED frames [own_fa, own_fb); the frames before and after are halo frames that a window's local
+ * problem may reach (h = floor(eps_time) of them on each side where a neighbour exists). Point i of the local problem
+ * has the global index index_base + i (components are keyed by it). min_frames 0 = the T4 rules, >= 1 = the
+ * PointCloudWorkF variant (eps_time <= 30). core uint8[frame_off_host[n_frames]] spans the whole local problem; the
+ * hint and its flag work as in rb_stdbscan_windowed. The multi-GPU recording (sharded.py, ShardedRecording) runs them on
+ * every rank with the halo exchanges and the stitch of all ranks' windows in between:
+ *   _pass_cores   the exact core flags of the owned points into core (clears the hint flag of the context)
+ *   _pass_keys    after the halo slots of core hold their owners' flags: windows [first_window, first_window + n_encode)
+ *                 encode their zones in rb_shard_pack_keys' format into vec int64[n_encode * (9 + 2 cap_keys)] (window k
+ *                 at (k - first_window) (9 + 2 cap_keys); entries beyond cap_keys are dropped, the counts stay true). The
+ *                 left zones of the first window and the right zones of the last one are encoded when left_neighbour /
+ *                 right_neighbour say that a neighbour holds the frames beyond. hint_outside (device, optional): the hint
+ *                 flag of passes 1 and 2 is OR-ed into it.
+ *   _pass_labels  with the stitched table (host: sorted keys, their ids) and, for min_frames, every cluster's start (host
+ *                 int64[n_start], its smallest global core index): labels int32 of the owned points (labels[0] = the
+ *                 first owned point). Syncs; fails with RB_ERR_ARG when the hint missed a point.
+ * None but _pass_labels syncs. RB_ERR_ARG before any work when the ids, offsets, owned range or cuts break the rules. */
+int rb_stdbscan_windowed_pass_cores(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                                    const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames, int64_t own_fa,
+                                    int64_t own_fb, const int64_t* cuts_host, int64_t n_windows, int64_t index_base, double eps_space,
+                                    float eps_time, int min_samples, int min_frames, const rb_stdbscan_hint* hint, uint8_t* core,
+                                    void* stream);
+int rb_stdbscan_windowed_pass_keys(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                                   const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames, int64_t own_fa,
+                                   int64_t own_fb, const int64_t* cuts_host, int64_t n_windows, int64_t index_base, double eps_space,
+                                   float eps_time, int min_samples, int min_frames, const rb_stdbscan_hint* hint, int left_neighbour,
+                                   int right_neighbour, const uint8_t* core, int64_t first_window, int64_t n_encode, int64_t cap_keys,
+                                   int64_t* vec, unsigned long long* hint_outside, void* stream);
+int rb_stdbscan_windowed_pass_labels(rb_ctx* ctx, const float* x, const float* y, const float* z, int64_t stride,
+                                     const int64_t* frame_off_host, const float* frame_ids_host, int64_t n_frames, int64_t own_fa,
+                                     int64_t own_fb, const int64_t* cuts_host, int64_t n_windows, int64_t index_base, double eps_space,
+                                     float eps_time, int min_samples, int min_frames, const rb_stdbscan_hint* hint, const uint8_t* core,
+                                     const int64_t* table_keys_host, const int32_t* table_ids_host, int64_t n_table,
+                                     const int64_t* start_of_host, int64_t n_start, int32_t* labels, void* stream);
+
 /* HOST function: the pairing of two run-length encodings of the SAME boundary points (rb_shard_pack_keys' zone format:
  * keys[j] holds from position starts[j] of the zone to the next start, -1 = not a core point; starts[0] = 0) into the
  * distinct (key_a, key_b) pairs of the core points, sorted. Cost follows the number of runs, not of points. Writes at

@@ -105,6 +105,14 @@ SIGNATURES = {
                                      C.POINTER(StdbscanHint), c_vp, c_vp, C.POINTER(c_i64), c_vp]),
     "rb_stdbscan_windowed_wf": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_f64, c_f32, c_i32, c_i32,
                                         C.POINTER(StdbscanHint), c_vp, c_vp, C.POINTER(c_i64), c_vp]),
+    "rb_stdbscan_windowed_pass_cores": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64,
+                                                c_f64, c_f32, c_i32, c_i32, C.POINTER(StdbscanHint), c_vp, c_vp]),
+    "rb_stdbscan_windowed_pass_keys": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64,
+                                               c_f64, c_f32, c_i32, c_i32, C.POINTER(StdbscanHint), c_i32, c_i32, c_vp, c_i64, c_i64,
+                                               c_i64, c_vp, c_vp, c_vp]),
+    "rb_stdbscan_windowed_pass_labels": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64,
+                                                 c_f64, c_f32, c_i32, c_i32, C.POINTER(StdbscanHint), c_vp, c_vp, c_vp, c_i64, c_vp,
+                                                 c_i64, c_vp, c_vp]),
     "rb_pair_zone_runs": (c_i64, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64]),
     "rb_comm_unique_id": (c_i32, [c_vp]),
     "rb_comm_init": (c_i32, [c_vp, c_vp, c_i32, c_i32]),

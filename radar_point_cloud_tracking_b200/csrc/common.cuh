@@ -51,12 +51,13 @@ enum rb_slot {
     RB_S_SHARD_IDS, RB_S_SHARD_LOCAL, RB_S_SHARD_KEYS,   // time-sharded driver: staged frame ids, local frame list, key flags / ranks
     RB_S_GROUP_TMP,         // rb_stable_group: frame offsets of its single frame
     RB_S_LAND_ORDERED,      // land accumulate, ordered path: cell ids, grouped intensities, segment table
-    RB_S_REC_FRAMES,        // windowed ST-DBSCAN: frame offsets, frame ids, hint-violation flag
+    RB_S_REC_FRAMES,        // windowed ST-DBSCAN: frame offsets, frame ids
     RB_S_REC_LOCAL,         // windowed ST-DBSCAN: times, global index, keys, labels, core flags of one window
     RB_S_REC_KEYS,          // windowed ST-DBSCAN: every window's run-length encoded zone keys
     RB_S_REC_KEYS_BIG,      // windowed ST-DBSCAN: encodings of the windows that outgrew the capacity guess
     RB_S_REC_TABLE,         // windowed ST-DBSCAN: the stitched key -> cluster id table
     RB_S_REC_CORE,          // windowed ST-DBSCAN: recording-wide core flags when the caller passes none
+    RB_S_REC_FLAG,          // windowed ST-DBSCAN: hint-violation flag, kept from pass 1 to pass 3
     RB_S_PLY_TILES,         // PLY formatter: bytes of each block of lines, then their scan
     RB_S_COUNT
 };

@@ -56,24 +56,31 @@ def check_frame_ids(ids: np.ndarray, after: Optional[int] = None) -> np.ndarray:
     return out
 
 
-def plan_windows(frame_off: np.ndarray, h: int, max_window_points: int) -> np.ndarray:
+def plan_windows(frame_off: np.ndarray, h: int, max_window_points: int, own: Optional[Sequence[int]] = None) -> np.ndarray:
     """Window cuts (frame indices ``0 = c_0 < ... < c_K = F``) for the frame-ordered points delimited by ``frame_off``
     (int64 [F+1]): one window when all points fit ``max_window_points``; otherwise windows of at least ``max(h, 1)``
     frames, each as long as its local problem (the window plus ``h`` frames on each side) stays within the budget. A
-    window whose minimum length already exceeds the budget is kept at that minimum."""
+    window whose minimum length already exceeds the budget is kept at that minimum.
+
+    ``own = (fa, fb)``: the windows cover only frames ``[fa, fb)`` (cuts from ``fa`` to ``fb``) while their local problems
+    may reach into the frames around them, which count against the budget - a rank's owned frames between its halos
+    (:class:`sharded.ShardedRecording`)."""
     off = np.asarray(frame_off, dtype=np.int64)
     F = len(off) - 1
     if F <= 0:
         raise RadarB200Error("a recording needs at least one frame")
-    if off[-1] <= max_window_points:
-        return np.array([0, F], dtype=np.int64)
+    fa0, fb0 = (0, F) if own is None else (int(own[0]), int(own[1]))
+    if not 0 <= fa0 < fb0 <= F:
+        raise RadarB200Error("the owned frames must be a non-empty range of the frames")
+    if off[-1] - off[0] <= max_window_points:
+        return np.array([fa0, fb0], dtype=np.int64)
     hmin = max(int(h), 1)
-    cuts = [0]
-    a = 0
-    while a < F:
+    cuts = [fa0]
+    a = fa0
+    while a < fb0:
         base = off[max(a - h, 0)]
-        # largest b in [a + hmin, F] with off[min(b + h, F)] - base <= budget (monotone in b)
-        lo, hi = min(a + hmin, F), F
+        # largest b in [a + hmin, fb0] with off[min(b + h, F)] - base <= budget (monotone in b)
+        lo, hi = min(a + hmin, fb0), fb0
         if off[min(lo + h, F)] - base <= max_window_points:
             while lo < hi:
                 mid = (lo + hi + 1) // 2
@@ -82,8 +89,8 @@ def plan_windows(frame_off: np.ndarray, h: int, max_window_points: int) -> np.nd
                 else:
                     hi = mid - 1
         b = lo
-        if 0 < F - b < hmin:                              # the rest would be too short: end this window earlier
-            b = F - hmin if F - hmin >= a + hmin else F
+        if 0 < fb0 - b < hmin:                            # the rest would be too short: end this window earlier
+            b = fb0 - hmin if fb0 - hmin >= a + hmin else fb0
         cuts.append(b)
         a = b
     return np.array(cuts, dtype=np.int64)
@@ -352,36 +359,16 @@ class RecordingDetection:
             chunks = self._chunks(raw_off)
             count = torch.zeros((nx, ny), dtype=torch.int32, device=d)
             isum = torch.zeros((nx, ny), dtype=torch.float64, device=d)
-            lib, h = self.ctx.lib, self.ctx.handle
             for ordered in (False, True):
-                entry = lib.rb_land_accumulate_ordered if ordered else lib.rb_land_accumulate
-                for fa, fb in chunks:                    # in block order: the ordered kernel continues from the stored sums
-                    a, b = int(raw_off[fa]), int(raw_off[fb])
-                    check(entry(h, ptr(xs[a:]), ptr(ys[a:]), ptr(iss[a:]), b - a, ptr(d_xe), nx + 1, ptr(d_ye), ny + 1, ptr(count),
-                                ptr(isum), stream_ptr()), "rb_land_accumulate")
+                self._land_accumulate(ordered, chunks, raw_off, d_xe, d_ye, count, isum)
                 if ordered:
                     break
-                flag = C.c_int32(0)
-                check(lib.rb_land_accumulate_status(h, C.byref(flag), stream_ptr()), "rb_land_accumulate_status")
-                if not flag.value:
+                if not self._land_inexact():
                     break
                 land_ordered = True
                 count.zero_(), isum.zero_()
             land = dev.land_cells(count, isum, built, cfg.land_persistence, cfg.land_min_intensity)
-            fx, fy, fi = (torch.empty(max(n_raw, 1), dtype=torch.float32, device=d) for _ in range(3))
-            fg = torch.empty(max(n_raw, 1), dtype=torch.int32, device=d)
-            f_off = np.zeros(F + 1, np.int64)
-            at = 0
-            for fa, fb in chunks:
-                a, b = int(raw_off[fa]), int(raw_off[fb])
-                loc_off = torch.from_numpy(raw_off[fa:fb + 1] - a).to(d)
-                out_off = torch.empty(fb - fa + 1, dtype=torch.int64, device=d)
-                check(lib.rb_land_filter(h, ptr(xs[a:]), ptr(ys[a:]), ptr(iss[a:]), ptr(gs[a:]), b - a, ptr(loc_off), fb - fa,
-                                         ptr(d_xe), nx + 1, ptr(d_ye), ny + 1, ptr(land), ptr(fx[at:]), ptr(fy[at:]), ptr(fi[at:]),
-                                         ptr(fg[at:]), ptr(out_off), None, stream_ptr()), "rb_land_filter")
-                o = out_off.cpu().numpy()
-                f_off[fa + 1:fb + 1] = o[1:] + at
-                at += int(o[-1])
+            fx, fy, fi, fg, f_off, at = self._land_filter(chunks, raw_off, d_xe, d_ye, land)
             pts = dev.PointBatch(fx, fy, fi, fg, torch.from_numpy(f_off).to(d), at)
             edges = (xe, ye)
         torch.cuda.current_stream(d).synchronize()
@@ -402,6 +389,46 @@ class RecordingDetection:
         return RecordingResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum, core=core, cuts=cuts,
                                frames_built=built, land_ordered=land_ordered, timings=timings,
                                frame_times=list(self._times) if self._csv_frames else None)
+
+    def _land_accumulate(self, ordered: bool, chunks, raw_off: np.ndarray, d_xe, d_ye, count, isum) -> None:
+        """``rb_land_accumulate`` (``ordered``: ``rb_land_accumulate_ordered``, continuing from the stored sums) over the
+        recording's chunks in block order."""
+        lib, h = self.ctx.lib, self.ctx.handle
+        xs, ys, iss, _ = self._store
+        entry = lib.rb_land_accumulate_ordered if ordered else lib.rb_land_accumulate
+        nx, ny = count.shape
+        for fa, fb in chunks:
+            a, b = int(raw_off[fa]), int(raw_off[fb])
+            check(entry(h, ptr(xs[a:]), ptr(ys[a:]), ptr(iss[a:]), b - a, ptr(d_xe), nx + 1, ptr(d_ye), ny + 1, ptr(count),
+                        ptr(isum), stream_ptr()), "rb_land_accumulate")
+
+    def _land_inexact(self) -> bool:
+        """Whether the accumulation since the last query saw a non-integer intensity (syncs; clears the flag)."""
+        flag = C.c_int32(0)
+        check(self.ctx.lib.rb_land_accumulate_status(self.ctx.handle, C.byref(flag), stream_ptr()), "rb_land_accumulate_status")
+        return bool(flag.value)
+
+    def _land_filter(self, chunks, raw_off: np.ndarray, d_xe, d_ye, land):
+        """``rb_land_filter`` of every chunk: the kept points ``(fx, fy, fi, fg)``, their frame offsets (host) and count."""
+        lib, h, d = self.ctx.lib, self.ctx.handle, self.device
+        xs, ys, iss, gs = self._store
+        n_raw, F = self._n, int(sum(len(o) - 1 for o in self._offs[1:]))
+        nx, ny = land.shape
+        fx, fy, fi = (torch.empty(max(n_raw, 1), dtype=torch.float32, device=d) for _ in range(3))
+        fg = torch.empty(max(n_raw, 1), dtype=torch.int32, device=d)
+        f_off = np.zeros(F + 1, np.int64)
+        at = 0
+        for fa, fb in chunks:
+            a, b = int(raw_off[fa]), int(raw_off[fb])
+            loc_off = torch.from_numpy(raw_off[fa:fb + 1] - a).to(d)
+            out_off = torch.empty(fb - fa + 1, dtype=torch.int64, device=d)
+            check(lib.rb_land_filter(h, ptr(xs[a:]), ptr(ys[a:]), ptr(iss[a:]), ptr(gs[a:]), b - a, ptr(loc_off), fb - fa,
+                                     ptr(d_xe), nx + 1, ptr(d_ye), ny + 1, ptr(land), ptr(fx[at:]), ptr(fy[at:]), ptr(fi[at:]),
+                                     ptr(fg[at:]), ptr(out_off), None, stream_ptr()), "rb_land_filter")
+            o = out_off.cpu().numpy()
+            f_off[fa + 1:fb + 1] = o[1:] + at
+            at += int(o[-1])
+        return fx, fy, fi, fg, f_off, at
 
     def _chunks(self, raw_off: np.ndarray):
         """Consecutive blocks grouped into frame ranges of fewer than 2^31 points (the land kernels' per-call limit)."""

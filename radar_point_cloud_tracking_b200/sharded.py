@@ -859,3 +859,371 @@ class ShardedDetection:
         out["h2d_bytes"] = t_echo.numel() * t_echo.element_size() + 3 * c.nbytes
         out["d2h_bytes"] = out["points"].nbytes + out["gains"].nbytes + out["labels"].nbytes + out["frame_off"].nbytes
         return out
+
+
+# ------------------------------------------------------------------------------------------ whole recordings
+def split_frames(n_frames: int, world: int, rank: int) -> Tuple[int, int]:
+    """Frames ``[a, b)`` of rank ``rank`` when ``n_frames`` frames are split into ``world`` contiguous shares whose sizes
+    differ by at most one (earlier ranks take the larger ones)."""
+    if world < 1 or not 0 <= rank < world or n_frames < 0:
+        raise RadarB200Error("split_frames: bad arguments")
+    q, r = divmod(int(n_frames), int(world))
+    a = rank * q + min(rank, r)
+    return a, a + q + (1 if rank < r else 0)
+
+
+def check_recording_stats(stats: np.ndarray, cluster: bool, h: int) -> None:
+    """The decisions of :meth:`ShardedRecording.finish` that can fail, taken from every rank's gathered
+    ``[frames, frames built, raw points, x_min, x_max, y_min, y_max, first id, last id]`` (``stats[world, 9]``): every rank
+    sees the same numbers, so all raise the same :class:`RadarB200Error` together and none is left in a collective."""
+    frames = stats[:, 0].astype(np.int64)
+    if int(frames.sum()) == 0:
+        raise RadarB200Error("finish() of an empty recording: no rank was fed any frame")
+    world = len(stats)
+    if cluster and world > 1:
+        need = max(int(h), 1)
+        short = [r for r in range(world) if frames[r] < need]
+        if short:
+            raise RadarB200Error(f"rank {short[0]} holds {int(frames[short[0]])} frames, fewer than the {need} that clustering over "
+                                 f"{world} ranks needs (max(floor(eps_time), 1)): give every rank at least {need} frames")
+        if h > 64:
+            raise RadarB200Error(f"an eps_time halo of {h} frames is more than the 64 frames the ranks exchange")
+    last, last_rank = None, None
+    for r in range(world):
+        if frames[r] == 0:
+            continue
+        first = int(stats[r, 7])
+        if last is not None and first <= last:
+            raise RadarB200Error(f"frame ids must increase strictly across ranks: rank {r}'s first id {first} is not above rank "
+                                 f"{last_rank}'s last id {last}")
+        last, last_rank = int(stats[r, 8]), r
+
+
+def window_payload(head: np.ndarray, entries: Sequence[np.ndarray]) -> np.ndarray:
+    """One rank's window encodings as one int64 vector for the all-gather: ``[n_windows | heads (9 per window) | per window
+    its keys, then its starts]``; ``head[k]`` = window k's 5 running entry counts and 4 zone lengths
+    (``rb_stdbscan_windowed_pass_keys``), ``entries`` = per window its keys and its starts (``head[k, 4]`` each)."""
+    head = np.asarray(head, np.int64).reshape(-1, 9)
+    return np.concatenate([[len(head)], head.ravel()] + [np.asarray(e, np.int64) for e in entries]).astype(np.int64)
+
+
+def stitch_windows(payloads: np.ndarray) -> Tuple[np.ndarray, np.ndarray, int]:
+    """The key -> cluster id table of a recording whose windows are spread over the ranks: ``payloads[r]`` = rank r's
+    :func:`window_payload` (zero padded). The global window list is all ranks' windows in rank order; every pair of
+    adjacent windows - inside a rank or across a rank edge - shares two boundary zones (own last frames | the next's left
+    halo, right halo | the next's own first frames), whose encodings are paired (:func:`pair_zone_runs`) and stitched
+    (:func:`stitch_components`). Every rank computes the same table from the same payloads."""
+    heads, runs, all_keys = [], [], []
+    for p in np.asarray(payloads, np.int64):
+        nw = int(p[0])
+        hr = p[1:1 + 9 * nw].reshape(nw, 9)
+        at = 1 + 9 * nw
+        for k in range(nw):
+            tot = int(hr[k, 4])
+            keys, starts = p[at:at + tot], p[at + tot:at + 2 * tot]
+            at += 2 * tot
+            bnd = np.concatenate([[0], hr[k, :5]])
+            runs.append([(keys[bnd[z]:bnd[z + 1]], starts[bnd[z]:bnd[z + 1]]) for z in range(4)])
+            all_keys.append(keys[bnd[4]:bnd[5]])
+            heads.append(hr[k])
+    e = np.zeros(0, np.int64)
+    segs = [[e, e, e, e] for _ in heads]
+    for k in range(len(heads) - 1):
+        for za, zb in ((2, 0), (3, 1)):                          # own last | next's left halo, right halo | next's own first
+            if heads[k][5 + za] != heads[k + 1][5 + zb]:
+                raise RadarB200Error("stitch: boundary zones of neighbouring windows do not match")
+            segs[k][za], segs[k + 1][zb] = pair_zone_runs(*runs[k][za], *runs[k + 1][zb])
+    tk, ti, ncl = stitch_components(segs, all_keys)
+    return np.ascontiguousarray(tk, np.int64), np.ascontiguousarray(ti, np.int32), int(ncl)
+
+
+def cluster_starts(table_keys: np.ndarray, table_ids: np.ndarray, n_clusters: int) -> np.ndarray:
+    """min_frames: every cluster's start, its smallest core index = the first key of its id in the sorted table."""
+    start_of = np.full(max(int(n_clusters), 1), -1, np.int64)
+    if len(table_ids):
+        uid, first = np.unique(table_ids, return_index=True)
+        start_of[uid] = np.asarray(table_keys)[first]
+    return start_of
+
+
+class ShardedRecording:
+    """One recording detected over several GPUs, one process per GPU (DESIGN.md section 3.11): rank r is fed a contiguous
+    share of the recording's frames - all of rank r's frames come before rank r+1's, ids increase strictly across ranks -
+    through the feeding calls of :class:`recording.RecordingDetection` (``add_block``, ``add_host_block``,
+    ``add_csv_frames``; each rank parses its own share of a CSV tree). :meth:`finish` is a collective that returns every
+    rank's :class:`recording.RecordingResult` for its own frames.
+
+    The results of all ranks, concatenated in rank order, equal ``RecordingDetection.finish()`` of one process fed the same
+    frames in the same order, bit for bit and id for id: raw and filtered points with their frame offsets; the land grid,
+    sums and mask (identical on every rank); ``land_ordered``; labels, core flags and the global ``n_clusters``;
+    ``frames_built`` (the recording's). Also with ``DetectionConfig.min_frames`` and ``cluster_3d``. ``world == 1`` is
+    exactly :class:`recording.RecordingDetection`.
+
+    Every collective goes through the engine (:class:`CudaEngine`: NCCL by the library; a test engine may swap them),
+    one communicator per rank, in one fixed order on every rank."""
+
+    def __init__(self, config=None, rank: Optional[int] = None, world: Optional[int] = None, group=None, engine=None,
+                 max_window_points: Optional[int] = None):
+        from .recording import RecordingDetection
+
+        self.group = group
+        self.rank = dist.get_rank(group) if rank is None else int(rank)
+        self.world = dist.get_world_size(group) if world is None else int(world)
+        if not 0 <= self.rank < self.world:
+            raise RadarB200Error(f"rank {self.rank} of a world of {self.world}")
+        self.engine = engine or CudaEngine()
+        self.engine.attach(self.rank, self.world, group)
+        self.device = self.engine.device
+        self.rec = RecordingDetection(config, self.device.index, max_window_points)
+        self.cfg = self.rec.cfg
+        self._key_cap = 1 << 15
+        self._pinned = None
+        self.timings = self.rec.timings
+
+    # ---- feeding: RecordingDetection's calls on this rank's share -----------------------------------------------------
+    def add_block(self, echo, cos_tab, sin_tab, range_res, frame_ids: Sequence[int]) -> None:
+        """:meth:`recording.RecordingDetection.add_block` for the next frames of this rank's share."""
+        self.rec.add_block(echo, cos_tab, sin_tab, range_res, frame_ids)
+
+    def add_host_block(self, echo, angle_units, scale, frame_ids: Sequence[int]) -> None:
+        """:meth:`recording.RecordingDetection.add_host_block` for the next frames of this rank's share."""
+        self.rec.add_host_block(echo, angle_units, scale, frame_ids)
+
+    def add_csv_frames(self, frame_files, frame_ids: Optional[Sequence[int]] = None, **kw) -> None:
+        """:meth:`recording.RecordingDetection.add_csv_frames` for the next frames of this rank's share: each rank parses
+        its own files. Pass ``frame_ids`` on every rank but the first (the default ids start at 0 on every rank)."""
+        self.rec.add_csv_frames(frame_files, frame_ids, **kw)
+
+    @property
+    def pipe(self):
+        return self.rec.pipe
+
+    @property
+    def csv_files(self):
+        return self.rec.csv_files
+
+    # ---- host read-backs and small all-gathers ------------------------------------------------------------------------
+    def _read(self, *tensors) -> list:
+        """Device tensors -> host numpy copies through one pinned buffer of this recording (grown, never shrunk), one sync."""
+        sizes = [t.numel() * t.element_size() for t in tensors]
+        total = sum((s + 15) // 16 * 16 for s in sizes)
+        if self._pinned is None or self._pinned.numel() < total:
+            self._pinned = torch.empty(max(total, 4096), dtype=torch.uint8, pin_memory=True)
+        views, at = [], 0
+        for t, s in zip(tensors, sizes):
+            v = self._pinned[at:at + s].view(t.dtype).view(t.shape)
+            v.copy_(t, non_blocking=True)
+            views.append(v)
+            at += (s + 15) // 16 * 16
+        torch.cuda.current_stream(self.device).synchronize()
+        return [np.array(v.numpy()) for v in views]
+
+    def _gather(self, vec: np.ndarray) -> np.ndarray:
+        """One host vector per rank (same length everywhere) -> ``[world, len]`` on every rank."""
+        return self._read(self.engine.all_gather(self.engine.upload(np.ascontiguousarray(vec))))[0]
+
+    # ---- the recording ------------------------------------------------------------------------------------------------
+    def finish(self, cluster: bool = True):
+        """Collective: land grid and filter over all ranks' frames, one ST-DBSCAN labelling of the recording whose
+        windows are spread over the ranks; this rank's :class:`recording.RecordingResult` (see the class docstring)."""
+        if self.world == 1:
+            return self.rec.finish(cluster)
+        return self._finish_protocol(cluster)
+
+    def _finish_protocol(self, cluster: bool = True):
+        """The protocol of :meth:`finish`. It also runs at ``world == 1``, where every collective is the identity:
+        tools/run_sharded_recording.py measures its cost there next to :meth:`recording.RecordingDetection.finish`."""
+        import contextlib
+        import time
+
+        from . import device as dev
+        from .recording import RecordingResult
+
+        rec, cfg, eng, d = self.rec, self.cfg, self.engine, self.device
+        if rec._finished:
+            raise RadarB200Error("finish() was already called")
+        rec._finished = True
+        eng.prepare_slots(1, lambda k: contextlib.nullcontext())
+        timings = dict(rec.timings)
+        t0 = time.perf_counter()
+
+        # ---- 1. what every rank holds: every decision that can fail is taken from these gathered numbers -------------
+        ids = np.concatenate(rec._ids) if rec._ids else np.zeros(0, np.int64)
+        F = len(ids)
+        raw_off = np.concatenate([[0]] + [o[1:] + b for o, b in zip(rec._offs[1:], rec._bases)]).astype(np.int64)
+        n_raw = rec._n
+        if rec._store is None:
+            rec._grow(1)
+        xs, ys, iss, gs = rec._store
+        raw = dev.PointBatch(xs, ys, iss, gs, torch.from_numpy(raw_off).to(d), n_raw)
+        built_here = int(np.count_nonzero(np.diff(raw_off)))
+        b4 = rec._b4 if rec._b4 is not None else np.zeros(4, np.float32)
+        stats = self._gather(np.array([F, built_here, n_raw, *b4, ids[0] if F else 0, ids[-1] if F else 0], np.float64))
+        h = int(math.floor(np.float32(cfg.eps_time))) if cfg.eps_time >= 0 else 0
+        check_recording_stats(stats, cluster, h)
+        built, n_all = int(stats[:, 1].sum()), int(stats[:, 2].sum())
+        have = stats[stats[:, 2] > 0]
+        gb4 = (np.array([have[:, 3].min(), have[:, 4].max(), have[:, 5].min(), have[:, 6].max()], np.float32)
+               if len(have) else None)
+        timings["stats"] = time.perf_counter() - t0
+
+        # ---- 2. land: one grid over the recording, every rank's sums added up -------------------------------------------
+        t0 = time.perf_counter()
+        pts, land, edges, count, isum, land_ordered = raw, None, None, None, None, False
+        if cfg.land_filter and n_all > 0 and built > cfg.land_min_frames:
+            xe, ye = dev.arange_edges(gb4[0], gb4[1], cfg.land_resolution), dev.arange_edges(gb4[2], gb4[3], cfg.land_resolution)
+            if len(xe) < 2 or len(ye) < 2:
+                raise RadarB200Error("degenerate land grid")
+            nx, ny = len(xe) - 1, len(ye) - 1
+            d_xe, d_ye = eng.upload(xe), eng.upload(ye)
+            chunks = rec._chunks(raw_off) if n_raw else []
+            count = torch.zeros((nx, ny), dtype=torch.int32, device=d)
+            isum = torch.zeros((nx, ny), dtype=torch.float64, device=d)
+            rec._land_accumulate(False, chunks, raw_off, d_xe, d_ye, count, isum)
+            inexact = self._gather(np.array([1 if rec._land_inexact() else 0], np.int64))
+            if not inexact.any():
+                eng.all_reduce_grids(count, isum)                # sums of integers: exact in any order
+            else:
+                # non-integer intensities: the float64 sums depend on the order of addition. The ordered accumulation
+                # runs as a chain in rank order - each rank continues from the sums of all ranks before it - and one
+                # all-reduce adds the last rank's grids to zeros everywhere else, which is exact
+                land_ordered = True
+                count.zero_(), isum.zero_()
+                grids = [count.view(-1), isum.view(-1)]
+                none = [count.new_empty(0), isum.new_empty(0)]
+                if self.rank > 0:
+                    eng.exchange(none, none, grids, none)
+                rec._land_accumulate(True, chunks, raw_off, d_xe, d_ye, count, isum)
+                if self.rank < self.world - 1:
+                    eng.exchange(none, grids, none, none)
+                    count.zero_(), isum.zero_()
+                eng.all_reduce_grids(count, isum)
+            land = dev.land_cells(count, isum, built, cfg.land_persistence, cfg.land_min_intensity)
+            if n_raw:
+                fx, fy, fi, fg, f_off, at = rec._land_filter(chunks, raw_off, d_xe, d_ye, land)
+            else:
+                fx, fy, fi = (torch.empty(1, dtype=torch.float32, device=d) for _ in range(3))
+                fg, f_off, at = torch.empty(1, dtype=torch.int32, device=d), np.zeros(F + 1, np.int64), 0
+            pts = dev.PointBatch(fx, fy, fi, fg, torch.from_numpy(f_off).to(d), at)
+            edges = (xe, ye)
+        p_off = raw_off if pts is raw else pts.frame_off.cpu().numpy()
+        torch.cuda.current_stream(d).synchronize()
+        timings["land"] = time.perf_counter() - t0
+
+        labels = torch.empty(0, dtype=torch.int32, device=d)
+        core, cuts, n_clusters = None, None, 0
+        if cluster:
+            labels, core, cuts, n_clusters = self._cluster(pts, p_off, ids, h, gb4, timings)
+        return RecordingResult(ids, raw, pts, labels, n_clusters, land, edges, count, isum, core=core, cuts=cuts,
+                               frames_built=built, land_ordered=land_ordered, timings=timings,
+                               frame_times=list(rec._times) if rec._csv_frames else None)
+
+    def _cluster(self, pts: PointBatch, p_off: np.ndarray, ids: np.ndarray, h: int, gb4, timings: dict):
+        """Steps 3 and 4 of :meth:`finish`: halos, then the three windowed passes with the stitch of every rank's windows."""
+        import ctypes as C
+        import time
+
+        from ._lib import StdbscanHint, check, ptr, stream_ptr
+        from .recording import plan_windows
+
+        cfg, eng, d, rec = self.cfg, self.engine, self.device, self.rec
+        ctx = rec.ctx
+        t0 = time.perf_counter()
+        F = len(ids)
+        h = min(h, F)                                            # (more than F only at world 1, without neighbours)
+        n_own = int(p_off[-1])
+        # ---- 3. layout of every rank's boundary frames; the local problem [left halo | owned | right halo] ------------
+        meta = self._read(eng.all_gather(eng.pack_layout(pts.frame_off, ids, F, h)))[0]
+        if int(meta[:, 0].sum()) == 0:
+            return torch.empty(0, dtype=torch.int32, device=d), None, None, 0
+        lids = lcnt = rids = rcnt = np.zeros(0, np.int64)
+        if self.rank > 0 and h:                                  # left halo = the left neighbour's last h frames
+            m = meta[self.rank - 1]
+            lids, lcnt = m[2 + 2 * h:2 + 3 * h], m[2 + 3 * h:2 + 4 * h]
+        if self.rank < self.world - 1 and h:                     # right halo = the right neighbour's first h frames
+            m = meta[self.rank + 1]
+            rids, rcnt = m[2:2 + h], m[2 + h:2 + 2 * h]
+        nl, nr = int(lcnt.sum()), int(rcnt.sum())
+        n_loc = nl + n_own + nr
+        index_base = int(meta[:self.rank, 0].sum()) - nl
+        loc_off = np.ascontiguousarray(np.concatenate([[0], np.cumsum(np.concatenate([lcnt, np.diff(p_off), rcnt]))]), dtype=np.int64)
+        loc_ids = np.ascontiguousarray(np.concatenate([lids, ids, rids]), dtype=np.float32)
+        own_fa, own_fb = len(lids), len(lids) + F
+        lo_end, hi_start = int(p_off[h]), int(p_off[F - h])       # owned points [0, lo_end) go left, [hi_start, n_own) right
+        dims = 3 if cfg.cluster_3d else 2
+        src = [pts.x, pts.y, pts.inten][:dims]
+        loc = [torch.empty(max(n_loc, 1), dtype=torch.float32, device=d) for _ in range(dims)]
+        for t, s in zip(loc, src):
+            t[nl:nl + n_own].copy_(s[:n_own])
+        eng.exchange([s[:lo_end] for s in src], [s[hi_start:n_own] for s in src], [t[:nl] for t in loc],
+                     [t[nl + n_own:n_loc] for t in loc])
+        X, Y, Z = loc[0], loc[1], (loc[2] if dims == 3 else None)
+        torch.cuda.current_stream(d).synchronize()
+        timings["layout_halos"] = time.perf_counter() - t0
+
+        # ---- 4. this rank's windows over its owned frames; the three passes ----------------------------------------------
+        t0 = time.perf_counter()
+        cuts = np.ascontiguousarray(plan_windows(loc_off, h, rec.window_budget(n_loc), own=(own_fa, own_fb)), dtype=np.int64)
+        n_w = len(cuts) - 1
+        hint = None
+        if gb4 is not None and Z is None:                        # every point lies in the global raw bounds: no plan syncs
+            hint = StdbscanHint()
+            hint.lo[0], hint.hi[0], hint.lo[1], hint.hi[1] = (float(v) for v in gb4)
+            hint.times_integer = 1
+        mf = 0 if cfg.min_frames is None else int(cfg.min_frames)
+        lib, hd = ctx.lib, ctx.handle
+        common = (hd, ptr(X), ptr(Y), ptr(Z), 1, loc_off.ctypes.data, loc_ids.ctypes.data, len(loc_ids), own_fa, own_fb,
+                  cuts.ctypes.data, n_w, index_base, float(cfg.eps_space), float(np.float32(cfg.eps_time)), int(cfg.min_samples), mf,
+                  C.byref(hint) if hint is not None else None)
+        core = torch.empty(max(n_loc, 1), dtype=torch.uint8, device=d)
+        check(lib.rb_stdbscan_windowed_pass_cores(*common, ptr(core), stream_ptr()), "rb_stdbscan_windowed_pass_cores")
+        eng.exchange_cores(core[:n_loc], nl, n_own, nr, lo_end, hi_start)  # halo points take their owner's core flags
+        torch.cuda.current_stream(d).synchronize()
+        timings["pass_cores"] = time.perf_counter() - t0
+
+        t0 = time.perf_counter()
+        left, right = int(self.rank > 0), int(self.rank < self.world - 1)
+
+        def encode(k0, n_enc, cap, flag=None):
+            vec = torch.empty(n_enc * (9 + 2 * cap), dtype=torch.int64, device=d)
+            check(lib.rb_stdbscan_windowed_pass_keys(*common, left, right, ptr(core), k0, n_enc, cap, ptr(vec), ptr(flag), stream_ptr()),
+                  "rb_stdbscan_windowed_pass_keys")
+            return vec.view(n_enc, 9 + 2 * cap)
+
+        cap = self._key_cap
+        flag = torch.zeros(1, dtype=torch.int64, device=d)
+        vec = encode(0, n_w, cap, flag)
+        head, bad = self._read(vec[:, :9], flag)
+        rows = [(vec[k], cap) for k in range(n_w)]
+        for k in range(n_w):                                     # a window that outgrew the guess is encoded again alone
+            need = int(head[k, 4])
+            if need > cap:
+                rows[k] = (encode(k, 1, need)[0], need)
+        self._key_cap = min(max(self._key_cap, int(head[:, 4].max()) * 5 // 4), 1 << 22)
+        parts = []
+        for k, (row, c) in enumerate(rows):
+            tot = int(head[k, 4])
+            parts += [row[9:9 + tot], row[9 + c:9 + c + tot]]
+        ent = self._read(*parts) if parts else []
+        payload = window_payload(head, ent)
+        torch.cuda.current_stream(d).synchronize()
+        timings["pass_keys"] = time.perf_counter() - t0
+
+        # ---- every rank's window encodings (sizes first, then the payload), stitched identically on every rank ------------
+        t0 = time.perf_counter()
+        sizes = self._gather(np.array([len(payload), int(bad[0])], np.int64))
+        if sizes[:, 1].any():
+            raise RadarB200Error("sharded recording: the global raw bounds do not contain every point of a local problem "
+                                 f"(rank {int(np.nonzero(sizes[:, 1])[0][0])}); the result would be invalid")
+        width = int(sizes[:, 0].max())
+        got = self._gather(np.concatenate([payload, np.zeros(width - len(payload), np.int64)]))
+        tk, ti, ncl = stitch_windows(got)
+        start_of = cluster_starts(tk, ti, ncl) if mf else np.full(1, -1, np.int64)
+        timings["stitch"] = time.perf_counter() - t0
+
+        t0 = time.perf_counter()
+        labels = torch.empty(max(n_own, 1), dtype=torch.int32, device=d)
+        check(lib.rb_stdbscan_windowed_pass_labels(*common, ptr(core), tk.ctypes.data, ti.ctypes.data, len(tk), start_of.ctypes.data,
+                                                   ncl if mf else 0, ptr(labels), stream_ptr()), "rb_stdbscan_windowed_pass_labels")
+        timings["pass_labels"] = time.perf_counter() - t0
+        return labels[:n_own], core[nl:nl + n_own], cuts - own_fa, int(ncl)
